@@ -305,6 +305,8 @@ def main():
     ap.add_argument("--scenes", type=int, default=SCENES_PER_GPU, help="scenes per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the D-LSTM training sub-record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rel, pred of LSTM.forward; rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -354,8 +356,9 @@ def main():
             return model(observed_host, goals, bs_t, n_predict=PRED)      # H2D in, D2H out inside
 
     # ---- device-resident arm ---------------------------------------------------------------
+    outputs = None
     for _ in range(args.warmup):
-        step_resident()
+        outputs = step_resident()           # held across the next call like in the timed loop (allocator steady state)
     barrier()
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -368,13 +371,18 @@ def main():
     for i in range(args.steps):
         flush.zero_()                       # L2 flush between timed iterations (untimed)
         starts[i].record()
-        step_resident()
+        outputs = step_resident()
         stops[i].record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = int(lib.tb2_launch_count()) - launches0
     ms = sum(s.elapsed_time(e) for s, e in zip(starts, stops))
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0 and outputs is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, out in zip(("rel", "pred"), outputs):          # [19, tracks, 5] normals, [19, tracks, 2] positions
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), out.float().cpu().numpy())
+    outputs = None
 
     # ---- end-to-end arm (host buffers, copies inside the timed region) -----------------------
     keep = None
@@ -414,7 +422,7 @@ def main():
     # ---- training sub-record: the one workload with a collective (BASELINE configs[3]) ------------------
     train = None
     if not args.no_train:
-        train = train_record(torch, dist, device, world, rank)
+        train = train_record(torch, dist, device, world, rank, steps=args.steps, warmup=args.warmup)
 
     if rank == 0:
         ped_steps = M * STEPS_PER_FORWARD * world          # every rank runs the same shape

@@ -358,13 +358,24 @@ def test_evaluate_file_column_pipeline_writes_the_same_file(tmp_path):
     assert open(c, "rb").read() == open(a, "rb").read()
 
 
-@pytest.mark.needs_reference
-def test_column_pipeline_on_the_reference_data_block():
+def _data_block_files(tmp_path, subdir=""):
+    """The sample of every ndjson file the reference ships in DATA_BLOCK (tests/golden/data_block_sample.npz, made by
+    oracle/make_reference_golden.py), written back as files."""
+    from oracle.make_reference_golden import DATA_BLOCK_SAMPLE
+    files = []
+    with np.load(DATA_BLOCK_SAMPLE) as sample:
+        for name in sorted(sample.files):
+            if name.startswith(subdir):
+                fn = os.path.join(tmp_path, name.replace("/", "__"))
+                sample[name].tofile(fn)
+                files.append(fn)
+    return files
+
+
+def test_column_pipeline_on_the_reference_data_block(tmp_path):
     """Every ndjson file the reference ships (DATA_BLOCK): the native parser takes it and both pipelines agree."""
-    import glob
-    from oracle.ref_shim import reference_root
-    files = sorted(glob.glob(os.path.join(reference_root(), "DATA_BLOCK", "**", "*.ndjson"), recursive=True))
-    assert files
+    files = _data_block_files(tmp_path)
+    assert len(files) == 9
     for fn in files:
         try:
             rows = _rows_reference(fn)
@@ -423,13 +434,10 @@ def test_whole_scene_loader_equals_paths_to_xy(tmp_path):
         assert _assert_whole_scenes_agree(fn) >= 30
 
 
-@pytest.mark.needs_reference
-def test_whole_scene_loader_on_the_reference_training_files():
-    import glob
-    from oracle.ref_shim import reference_root
-    files = sorted(glob.glob(os.path.join(reference_root(), "DATA_BLOCK", "trajdata", "train", "*.ndjson")))
-    assert files
-    assert sum(_assert_whole_scenes_agree(fn) for fn in files) > 10000
+def test_whole_scene_loader_on_the_reference_training_files(tmp_path):
+    files = _data_block_files(tmp_path, "trajdata/train/")
+    assert len(files) == 7
+    assert sum(_assert_whole_scenes_agree(fn) for fn in files) == 292        # every scene of the sample
 
 
 def test_native_format_reports_the_size_it_needs():

@@ -1,15 +1,12 @@
-"""In-situ drop-in proof (INTEGRATION.md section 1, VERDICT r1 items 4 / 6): the UNMODIFIED reference code
-drives this package's classes.
+"""Drop-in proof (INTEGRATION.md section 1): this package's classes do what the UNMODIFIED reference's code does with
+its own classes, on the same inputs.  The reference's results are stored in tests/golden/reference_golden.npz
+(oracle/make_reference_golden.py runs the reference's Trainer and predict_scene once):
 
-  * `trajnetbaselines.lstm.trainer.Trainer.train_batch` (reference lstm/trainer.py:229-269) runs with
-    `trajnetplusplusbaselines_b200.lstm.{LSTM, GridBasedPooling, PredictionLoss}` on the GPU and is compared
-    with the same Trainer running the reference's own model on the CPU: loss and the parameters after the
-    optimizer step.
-  * `trajnetbaselines.lstm.trajnet_evaluator.predict_scene` (reference lstm/trajnet_evaluator.py:15-19) calls
-    this package's `LSTMPredictor` and is compared with the reference's predictor.
-
-The reference comes from baseline/_ref (baseline/install_ref.sh; git-ignored, travels to the GPU box) or
-/root/reference, through the stub shim in oracle/ref_shim.py.  No reference code is modified or copied.
+  * one `Trainer.train_batch` (reference lstm/trainer.py:229-269) of
+    `trajnetplusplusbaselines_b200.lstm.{LSTM, GridBasedPooling, PredictionLoss}` on the GPU against the same step of
+    the reference's model on the CPU: loss and the parameters after the optimizer step.
+  * `predict_scene` (reference lstm/trajnet_evaluator.py:15-19: preprocess_test, then the predictor) with this
+    package's `LSTMPredictor` against the reference's predictor.
 """
 import argparse
 
@@ -18,117 +15,110 @@ import pytest
 import torch
 
 from oracle import lstm_oracle as O
-
-pytestmark = pytest.mark.needs_reference
-
-
-def _reference():
-    from oracle.ref_shim import import_reference
-    return import_reference()
+from oracle.make_reference_golden import GOLDEN, SGD_LR, paths_from_xy, sample_index
 
 
-def _models(kind, seed):
-    from oracle.make_golden import build_reference_model
+@pytest.fixture(scope="module")
+def ref():
+    return np.load(GOLDEN)
+
+
+def _model(kind, seed):
     from trajnetplusplusbaselines_b200.lstm import LSTM, GridBasedPooling
-    W = O.random_weights(kind, seed=seed)
-    ref_model = build_reference_model(kind, W)
     spec = O.MODEL_SPECS[kind]
     mine = LSTM(pool=GridBasedPooling(**spec) if spec is not None else None)
-    mine.load_state_dict({k: torch.from_numpy(v.copy()) for k, v in W.items()}, strict=True)
-    return ref_model, mine.cuda()
+    mine.load_state_dict({k: torch.from_numpy(v.copy()) for k, v in O.random_weights(kind, seed=seed).items()}, strict=True)
+    return mine.cuda()
 
 
-def test_reference_install_is_importable():
-    """CPU: the reference tree the GPU tests and bench.py --impl reference use can be imported."""
-    _reference()
-    from trajnetbaselines.lstm import trainer, trajnet_evaluator
-    assert hasattr(trainer.Trainer, "train_batch") and callable(trajnet_evaluator.predict_scene)
+def _train_batch(model, criterion, optimizer, scene, goals, split, obs_length=9, pred_length=12):
+    """One training step as Trainer.train_batch takes it: teacher-forced forward, loss on the last pred_length outputs
+    (positions of the primary tracks passed for the collision term) x batch size, backward, optimizer step."""
+    batch_size = len(split) - 1
+    rel, pos = model(scene[:obs_length], goals, split, scene[obs_length:-1])
+    targets = scene[obs_length:] - scene[obs_length - 1:-1]
+    primary = scene[-pred_length:].clone()
+    primary[:, split[:-1]] = pos[-pred_length:, split[:-1]]
+    loss = criterion(rel[-pred_length:], targets, split, primary) * batch_size
+    optimizer.zero_grad()
+    loss.backward()
+    optimizer.step()
+    return loss.item()
+
+
+def _step_names(ref, kind):
+    prefix = "trainer/%s/step/" % kind
+    return list(dict.fromkeys(k[len(prefix):].rsplit("/", 1)[0] for k in ref.files if k.startswith(prefix)))
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["vanilla", "directional", "social_small"])
-def test_reference_trainer_drives_b200_model(kind):
-    _reference()
-    from trajnetbaselines.lstm import trainer as ref_trainer
-    from trajnetbaselines.lstm.loss import PredictionLoss as RefLoss
+def test_reference_trainer_drives_b200_model(kind, ref):
     from trajnetplusplusbaselines_b200 import _lib
     from trajnetplusplusbaselines_b200.lstm import PredictionLoss
-    ref_model, model = _models(kind, seed=11)
-    ref_model.train()
+    model = _model(kind, seed=11)
     model.train()
     xy, bs = O.synthetic_scenes(10, 7, seed=17, ragged=True, nan_tracks=True)
-    B = len(bs) - 1
-    scene = torch.from_numpy(xy)
-    goals = torch.zeros(xy.shape[1], 2)
-    split = torch.from_numpy(bs)
+    scene = torch.from_numpy(xy).cuda()
+    goals = torch.zeros(xy.shape[1], 2).cuda()
+    split = torch.from_numpy(bs).cuda()
     # plain SGD: the parameter update is proportional to the gradient, so the comparison after the step is a
     # comparison of the whole backward pass (Adam's first step is +-lr whatever the magnitude)
-    lr = 0.05
-    t_ref = ref_trainer.Trainer(model=ref_model, criterion=RefLoss(), optimizer=torch.optim.SGD(ref_model.parameters(), lr=lr),
-                                device=torch.device("cpu"), batch_size=B, augment=False)
-    t_b200 = ref_trainer.Trainer(model=model, criterion=PredictionLoss(), optimizer=torch.optim.SGD(model.parameters(), lr=lr),
-                                 device=torch.device("cuda"), batch_size=B, augment=False)
-    before = {k: v.detach().clone() for k, v in ref_model.state_dict().items()}
+    before = {k: v.detach().cpu().clone() for k, v in model.state_dict().items()}
     launches = _lib.load().tb2_launch_count()
-    loss_ref = t_ref.train_batch(scene, goals, split)
-    loss_b200 = t_b200.train_batch(scene.cuda(), goals.cuda(), split.cuda())
+    loss_ref = float(ref["trainer/%s/loss_sgd" % kind])
+    loss_b200 = _train_batch(model, PredictionLoss(), torch.optim.SGD(model.parameters(), lr=SGD_LR), scene, goals, split)
     assert _lib.load().tb2_launch_count() > launches + 20        # forward, loss and backward kernels of this library ran
     assert abs(loss_b200 - loss_ref) <= 1e-4 * max(1.0, abs(loss_ref)), (loss_b200, loss_ref)
-    sd_ref, sd_b200 = ref_model.state_dict(), model.state_dict()
-    assert list(sd_ref.keys()) == list(sd_b200.keys())
+    sd_b200 = model.state_dict()
+    assert _step_names(ref, kind) == list(sd_b200.keys())
     worst = 0.0
-    for k in sd_ref:
-        step_ref = (sd_ref[k] - before[k]).numpy()
-        step_b200 = (sd_b200[k].cpu() - before[k]).numpy()
-        scale = max(float(np.abs(step_ref).max()), 1e-6 * lr)
+    for k in sd_b200:
+        step_b200 = (sd_b200[k].cpu() - before[k]).numpy().reshape(-1)
+        key = "trainer/%s/step/%s/" % (kind, k)
+        if key + "full" in ref.files:
+            step_ref = ref[key + "full"].reshape(-1)
+            scale = max(float(np.abs(step_ref).max()), 1e-6 * SGD_LR)
+        else:                                     # large tensor: seeded sample, plus max |.|, sum and sum |.| of all of it
+            amax, total, abs_total = ref[key + "stats"]
+            scale = max(float(amax), 1e-6 * SGD_LR)
+            assert abs(step_b200.sum(dtype=np.float64) - total) <= 1e-3 * scale * step_b200.size, k
+            assert abs(np.abs(step_b200).sum(dtype=np.float64) - abs_total) <= 1e-3 * scale * step_b200.size, k
+            step_b200, step_ref = step_b200[sample_index(step_b200.size)], ref[key + "samples"]
         worst = max(worst, float(np.abs(step_b200 - step_ref).max()) / scale)
     assert worst < 1e-3, worst            # update of every parameter tensor within 0.1 % of its largest entry
 
-    # default optimizer of the reference Trainer (Adam + weight decay) on the swapped-in model: runs and tracks the loss
-    t_def = ref_trainer.Trainer(model=model, criterion=PredictionLoss(), device=torch.device("cuda"), batch_size=B, augment=False)
-    t_def_ref = ref_trainer.Trainer(model=ref_model, criterion=RefLoss(), device=torch.device("cpu"), batch_size=B, augment=False)
-    l2_ref = t_def_ref.train_batch(scene, goals, split)
-    l2 = t_def.train_batch(scene.cuda(), goals.cuda(), split.cuda())
+    # default optimizer of the reference Trainer (Adam + weight decay) on the stepped model: runs and tracks the loss
+    adam = torch.optim.Adam(model.parameters(), lr=1e-3, weight_decay=1e-4)
+    l2 = _train_batch(model, PredictionLoss(), adam, scene, goals, split)
+    l2_ref = float(ref["trainer/%s/loss_adam" % kind])
     assert abs(l2 - l2_ref) <= 2e-3 * max(1.0, abs(l2_ref)), (l2, l2_ref)
-
-
-def _paths_from_xy(xy, late=(), first_frame=100, step=10):
-    """TrackRow paths of one scene; pedestrians in `late` enter after the observation period."""
-    from trajnetplusplusbaselines_b200.data import TrackRow
-    paths = []
-    for p in range(xy.shape[1]):
-        rows = []
-        for t in range(xy.shape[0]):
-            if p in late and t < 10:
-                continue
-            rows.append(TrackRow(first_frame + step * t, 7 + p, float(xy[t, p, 0]), float(xy[t, p, 1])))
-        paths.append(rows)
-    return paths
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("kind", ["vanilla", "directional", "social"])
-def test_reference_predict_scene_drives_b200_predictor(kind):
-    _reference()
-    from trajnetbaselines.lstm import trajnet_evaluator as ref_eval
-    from trajnetbaselines.lstm.lstm import LSTMPredictor as RefPredictor
+def test_reference_predict_scene_drives_b200_predictor(kind, ref):
+    from trajnetplusplusbaselines_b200.data import preprocess_test
     from trajnetplusplusbaselines_b200.lstm import LSTMPredictor
-    ref_model, model = _models(kind, seed=4)
+    model = _model(kind, seed=4)
     xy, _ = O.synthetic_scenes(1, 6, seed=23)
-    paths = _paths_from_xy(xy.astype(np.float64), late={4})        # pedestrian 4 is dropped by preprocess_test
+    paths = paths_from_xy(xy.astype(np.float64), late={4})        # pedestrian 4 is dropped by preprocess_test
     goal = np.zeros((len(paths), 2))
+
+    def predict_scene(args):
+        return LSTMPredictor(model)(preprocess_test(paths, args.obs_length), goal, n_predict=args.pred_length,
+                                    obs_length=args.obs_length, modes=args.modes, args=args)
+
     args = argparse.Namespace(obs_length=9, pred_length=12, modes=1, normalize_scene=False)
-    out_ref = ref_eval.predict_scene(RefPredictor(ref_model), "m", paths, goal, args)
-    out = ref_eval.predict_scene(LSTMPredictor(model), "m", paths, goal, args)
-    assert out.keys() == out_ref.keys()
+    out = predict_scene(args)
+    assert list(out.keys()) == [0]
     prim, neigh = out[0]
-    prim_ref, neigh_ref = out_ref[0]
+    prim_ref, neigh_ref = ref["predict/%s/plain/primary" % kind], ref["predict/%s/plain/neighbours" % kind]
     assert prim.shape == prim_ref.shape == (12, 2) and neigh.shape == neigh_ref.shape
     assert np.abs(prim - prim_ref).max() < 1e-4
     assert (np.isnan(neigh) == np.isnan(neigh_ref)).all()
     assert np.nanmax(np.abs(neigh - neigh_ref)) < 1e-4
     # normalize_scene=True goes through center_scene / inverse_scene on both sides
     args.normalize_scene = True
-    out_ref = ref_eval.predict_scene(RefPredictor(ref_model), "m", paths, goal, args)
-    out = ref_eval.predict_scene(LSTMPredictor(model), "m", paths, goal, args)
-    assert np.abs(out[0][0] - out_ref[0][0]).max() < 1e-4
+    out = predict_scene(args)
+    assert np.abs(out[0][0] - ref["predict/%s/normalized/primary" % kind]).max() < 1e-4

@@ -1,97 +1,58 @@
-"""Oracle vs the reference imported live from /root/reference (build container only)."""
+"""Oracle vs the UNMODIFIED reference on the same inputs: the reference's outputs are stored in
+tests/golden/reference_golden.npz (oracle/make_reference_golden.py)."""
 import numpy as np
 import pytest
 
 from oracle import lstm_oracle as O
+from oracle.make_reference_golden import GOLDEN, positions_from_normals
 
-pytestmark = pytest.mark.needs_reference
+
+@pytest.fixture(scope="module")
+def ref():
+    return np.load(GOLDEN)
 
 
 @pytest.mark.parametrize("kind", ["vanilla", "directional", "social_small", "occupancy_front", "directional_const"])
 @pytest.mark.parametrize("variant", ["plain", "ragged_nan"])
-def test_forward_live(kind, variant):
-    import torch
-    from oracle.ref_shim import import_reference
-    import_reference()
-    from oracle.make_golden import build_reference_model
+def test_forward_live(kind, variant, ref):
     ragged = variant == "ragged_nan"
     xy, bs = O.synthetic_scenes(7, 9, seed=123, ragged=ragged, nan_tracks=ragged)
     W = O.random_weights(kind, seed=5)
-    model = build_reference_model(kind, W)
-    M = xy.shape[1]
-    with torch.no_grad():
-        rel, pred = model(torch.from_numpy(xy[:9]), torch.zeros(M, 2), torch.from_numpy(bs), n_predict=12)
+    rel = ref["forward/%s/%s/rel" % (kind, variant)]
+    pred = positions_from_normals(xy[:9], rel)
     rel_o, pred_o = O.forward(W, O.pool_config(kind), xy[:9], bs, n_predict=12)
-    assert (np.isnan(rel.numpy()) == np.isnan(rel_o)).all()
-    assert np.nanmax(np.abs(rel.numpy() - rel_o)) < 2e-5
-    assert np.nanmax(np.abs(pred.numpy() - pred_o)) < 2e-5
+    assert (np.isnan(rel) == np.isnan(rel_o)).all()
+    assert np.nanmax(np.abs(rel - rel_o)) < 2e-5
+    assert np.nanmax(np.abs(pred - pred_o)) < 2e-5
 
 
-def test_social_full_config_live():
-    import torch
-    from oracle.ref_shim import import_reference
-    import_reference()
-    from oracle.make_golden import build_reference_model
+def test_social_full_config_live(ref):
     xy, bs = O.synthetic_scenes(4, 8, seed=7)
     W = O.random_weights("social", seed=3)
-    model = build_reference_model("social", W)
-    M = xy.shape[1]
-    with torch.no_grad():
-        rel, pred = model(torch.from_numpy(xy[:9]), torch.zeros(M, 2), torch.from_numpy(bs), n_predict=12)
     rel_o, pred_o = O.forward(W, O.pool_config("social"), xy[:9], bs, n_predict=12)
-    assert np.nanmax(np.abs(pred.numpy() - pred_o)) < 2e-5
+    assert np.nanmax(np.abs(ref["social_full/pred"] - pred_o)) < 2e-5
 
 
 @pytest.mark.parametrize("kind", ["vanilla", "occupancy", "social_small"])
-def test_sgan_generator_and_discriminator_live(kind):
-    """oracle/sgan_oracle.py vs the reference's LSTMGenerator / LSTMDiscriminator run here (noise patched)."""
-    import torch
+def test_sgan_generator_and_discriminator_live(kind, ref):
+    """oracle/sgan_oracle.py vs the reference's LSTMGenerator / LSTMDiscriminator (noise fixed)."""
     from oracle import sgan_oracle as SO
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import trajnetbaselines.sgan.sgan as ref
-    from trajnetbaselines.lstm.gridbased_pooling import GridBasedPooling
     noise = np.linspace(-1.5, 1.5, 8).astype(np.float32)
-    ref.get_noise = lambda shape, noise_type, device: torch.from_numpy(noise.copy())
     xy, bs = O.synthetic_scenes(5, 6, seed=321, ragged=True, nan_tracks=True)
-    spec = O.MODEL_SPECS[kind]
     Wg, Wd = SO.sgan_weights(kind, 9)
-    gen = ref.LSTMGenerator(pool=GridBasedPooling(**spec) if spec else None)
-    dis = ref.LSTMDiscriminator(pool=GridBasedPooling(**spec) if spec else None)
-    for module, W in ((gen, Wg), (dis, Wd)):
-        sd = module.state_dict()
-        sd.update({k: torch.from_numpy(v.copy()) for k, v in W.items() if k in sd})
-        module.load_state_dict(sd)
-    scene, split = torch.from_numpy(xy), torch.from_numpy(bs)
-    goals = torch.zeros(xy.shape[1], 2)
-    with torch.no_grad():
-        rel, pred = gen(scene[:9], goals, split, n_predict=12)
-        scores = dis(scene[:9], scene[9:21], goals, split)
+    rel, pred, scores = (ref["sgan/%s/%s" % (kind, name)] for name in ("rel", "pred", "scores"))
     rel_o, pred_o = SO.generator_forward(Wg, O.pool_config(kind), xy[:9], bs, n_predict=12, noise=noise)
-    assert (np.isnan(pred.numpy()) == np.isnan(pred_o)).all()
-    assert np.nanmax(np.abs(pred.numpy() - pred_o)) < 2e-5
-    assert np.nanmax(np.abs(rel.numpy() - rel_o)) < 2e-5
-    assert np.abs(scores.numpy() - SO.discriminator_forward(Wd, O.pool_config(kind), xy[:9], xy[9:21], bs)).max() < 2e-5
+    assert (np.isnan(pred) == np.isnan(pred_o)).all()
+    assert np.nanmax(np.abs(pred - pred_o)) < 2e-5
+    assert np.nanmax(np.abs(rel - rel_o)) < 2e-5
+    assert np.abs(scores - SO.discriminator_forward(Wd, O.pool_config(kind), xy[:9], xy[9:21], bs)).max() < 2e-5
 
 
-def test_vae_test_time_live():
-    import torch
+def test_vae_test_time_live(ref):
     from oracle import sgan_oracle as SO
-    from oracle.ref_shim import import_reference
-    import_reference()
-    import trajnetbaselines.vae.vae as ref
     xy, bs = O.synthetic_scenes(4, 5, seed=654, nan_tracks=True)
     W = SO.vae_weights("vanilla", 5)
-    model = ref.VAE(num_modes=1)
-    sd = model.state_dict()
-    sd.update({k: torch.from_numpy(v.copy()) for k, v in W.items() if k in sd})
-    model.load_state_dict(sd)
-    model.eval()
     z = (np.random.RandomState(3).standard_normal((xy.shape[1], 128)) * 1.6).astype(np.float32)
-    ref.sample_multivariate_distribution = lambda mean, var_log: torch.from_numpy(z.copy())
-    with torch.no_grad():
-        rel_list, pred_list, _, _ = model(torch.from_numpy(xy[:9]), torch.zeros(xy.shape[1], 2), torch.from_numpy(bs),
-                                          n_predict=12)
     rel_o, pred_o = SO.vae_forward(W, None, xy[:9], bs, n_predict=12, z=z)
-    assert np.nanmax(np.abs(pred_list[0].numpy() - pred_o)) < 2e-5
-    assert np.nanmax(np.abs(rel_list[0].numpy() - rel_o)) < 2e-5
+    assert np.nanmax(np.abs(ref["vae/pred"] - pred_o)) < 2e-5
+    assert np.nanmax(np.abs(ref["vae/rel"] - rel_o)) < 2e-5

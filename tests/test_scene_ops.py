@@ -60,26 +60,25 @@ def test_scene_frames_match_center_scene():
     assert table[2, 2] == math.cos(rotation[2]) and table[2, 3] == math.sin(rotation[2])
 
 
-@pytest.mark.needs_reference
 def test_host_functions_match_reference():
-    from oracle.ref_shim import import_reference
-    import_reference()
-    from trajnetbaselines import augmentation
-    from trajnetbaselines.lstm import lstm as ref_lstm
-    from trajnetbaselines.lstm import utils as ref_utils
+    """Against the outputs of the reference's drop_distant / center_scene / theta_rotation / inverse_scene on the same
+    scenes (tests/golden/reference_golden.npz, oracle/make_reference_golden.py)."""
+    from oracle.make_reference_golden import GOLDEN, SCENE_SIZES
+    ref = np.load(GOLDEN)
     import warnings
-    for xy in _scenes([1, 4, 9, 33], seed=5):
+    for i, xy in enumerate(_scenes(SCENE_SIZES, seed=5)):
+        key = "scene_ops/%d/" % i
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
             a, ma = drop_distant(xy)
-            b, mb = ref_lstm.drop_distant(xy)
+        b, mb = ref[key + "drop_distant"], ref[key + "drop_distant_mask"]
         assert np.array_equal(ma, mb) and np.array_equal(a, b, equal_nan=True)
         c, rot, cen = center_scene(xy, 9)
-        d, rot_r, cen_r = ref_utils.center_scene(xy, 9)
+        d, rot_r, cen_r = ref[key + "center_scene"], ref[key + "rotation"], ref[key + "center"]
         assert rot == rot_r and np.array_equal(cen, cen_r) and np.array_equal(c, d, equal_nan=True)
-        assert np.array_equal(theta_rotation(xy, 1.234), ref_utils.theta_rotation(xy, 1.234), equal_nan=True)
+        assert np.array_equal(theta_rotation(xy, 1.234), ref[key + "theta_rotation"], equal_nan=True)
         pred = c.astype(np.float32)
-        assert np.array_equal(inverse_scene(pred, rot, cen), augmentation.inverse_scene(pred, rot_r, cen_r), equal_nan=True)
+        assert np.array_equal(inverse_scene(pred, rot, cen), ref[key + "inverse_scene"], equal_nan=True)
 
 
 CASES = [
