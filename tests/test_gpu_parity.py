@@ -148,30 +148,6 @@ def test_pool_forward_matches_oracle(kind):
     assert maxdiff(out, ref) < TOL_STEP
 
 
-@pytest.mark.parametrize("kind", ["occupancy", "directional", "directional_const"])
-def test_pool_forward_dense_grid_variant(kind, monkeypatch):
-    """TB2_GRID_TC=1: the opt-in dense tcgen05 formulation of the occupancy / directional first Linear
-    (profiles/round2_grid_tc_experiment.txt) against the oracle."""
-    from trajnetplusplusbaselines_b200.lstm import GridBasedPooling
-    monkeypatch.setenv("TB2_GRID_TC", "1")
-    cfg = O.pool_config(kind)
-    W = O.random_weights(kind, seed=22)
-    rng = np.random.RandomState(6)
-    B, N = 7, 12
-    obs2 = (rng.randn(B, N, 2) * 2.0).astype(np.float32)
-    obs1 = obs2 - (rng.randn(B, N, 2) * 0.3).astype(np.float32)
-    hid = (rng.randn(B, N, 128) * 0.5).astype(np.float32)
-    obs2[2, 5:] = np.nan
-    obs1[2, 5:] = np.nan
-    obs1[3, 1] = np.nan
-    ref = O.pool_forward(cfg, W, hid, obs1, obs2)
-    pool = GridBasedPooling(**O.MODEL_SPECS[kind])
-    pool.load_state_dict({k[len("pool."):]: torch.from_numpy(v.copy()) for k, v in W.items() if k.startswith("pool.")}, strict=True)
-    pool = pool.cuda()
-    out = pool(torch.from_numpy(hid).cuda(), torch.from_numpy(obs1).cuda(), torch.from_numpy(obs2).cuda())
-    assert maxdiff(out, ref) < TOL_STEP
-
-
 # ---------------------------------------------------------------------------------------------
 # step and sequence
 # ---------------------------------------------------------------------------------------------

@@ -215,7 +215,6 @@ int tb2_lstm_create(const tb2_lstm_config* cfg, tb2_lstm** out) {
     m->C = 0; m->cells = 0; m->n_mlp = 0; m->P = 0; m->pool_out = 0;
     m->We = m->be = m->Wn = m->bn = m->WencT = m->benc = m->Wt1 = m->base1 = nullptr;
     m->Wt1_hi = m->Wt1_lo = m->Wt1_nat_hi = m->Wt1_nat_lo = m->Wt1_sw_hi = m->Wt1_sw_lo = nullptr;
-    m->W2_sw = nullptr;
     for (int i = 0; i < 2; ++i) { m->WgT[i] = m->bg[i] = nullptr; m->Wg_hi[i] = m->Wg_lo[i] = nullptr; }
     for (int i = 0; i < kMaxMlpLayers; ++i) { m->WT[i] = m->bl[i] = nullptr; m->W_hi[i] = m->W_lo[i] = nullptr; }
     m->mp_Ws = m->mp_bs = m->mp_Wv = m->mp_bv = m->mp_WhT = m->mp_bh = m->mp_WoT = m->mp_bo = nullptr;
@@ -378,26 +377,6 @@ int tb2_lstm_create(const tb2_lstm_config* cfg, tb2_lstm** out) {
                 ALLOC(sl, 4);
                 m->Wt1_sw_hi = sh;
                 m->Wt1_sw_lo = sl;
-                if (m->n_mlp == 2 && m->mlp_dims[2] == 256 && m->mlp_dims[1] % 32 == 0) {
-                    float* w2;
-                    ALLOC(w2, (size_t)m->mlp_dims[1] * 256);      // bf16 hi + lo of [256, d1]
-                    m->W2_sw = w2;
-                }
-            }
-        }
-        {
-            // occupancy / directional: first Linear as a dense 3-pass tcgen05 GEMM over an explicit (sparse, zero-padded)
-            // grid row per pedestrian: weights [d1][K padded to 64] in (cell, channel) order as bf16 (hi, lo)
-            const char* no_tc = getenv("TB2_DISABLE_TC");
-            const int k0p = (m->C * m->cells + 63) / 64 * 64;
-            if (cfg->pool_type != TB2_POOL_SOCIAL && m->n_mlp >= 1 && !(no_tc && no_tc[0] == '1') &&
-                dense_tc_supported(k0p, m->mlp_dims[1])) {
-                const size_t half = ((size_t)k0p * m->mlp_dims[1] + 1) / 2;
-                float *hi, *lo;
-                ALLOC(hi, half);
-                ALLOC(lo, half);
-                m->W_hi[0] = hi;
-                m->W_lo[0] = lo;
             }
         }
         for (int layer = 1; layer < m->n_mlp; ++layer) {

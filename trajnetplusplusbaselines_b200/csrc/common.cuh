@@ -130,10 +130,9 @@ struct tb2_lstm {
     void* Wt1_nat_lo;
     void* Wt1_sw_hi;       // social, C == 16: the same slabs as a SWIZZLE_32B shared-memory image (bulk-copy source of
     void* Wt1_sw_lo;       // sparse_layer1_pair)
-    void* W2_sw;           // social two_layer with 256 outputs: pool.embedding.2.weight as k-step bulk-copy images (fused layer 2)
     float* WT[tb2::kMaxMlpLayers];   // layers >= 2: [K, N] transposed
     float* bl[tb2::kMaxMlpLayers];   // biases of layers >= 2
-    void* W_hi[tb2::kMaxMlpLayers];  // bf16 [N, K] (hi, lo) split for the tcgen05 path (null: FFMA path)
+    void* W_hi[tb2::kMaxMlpLayers];  // layer 1 (the second Linear): bf16 [N, K] (hi, lo) split for the tcgen05 path (null: FFMA path)
     void* W_lo[tb2::kMaxMlpLayers];
     std::vector<cudaEvent_t> step_events;     // tb2_lstm_forward_sequence_host: one event per recurrence step
     // HiddenStateMLPPooling (TB2_POOL_HIDDEN_MLP)
@@ -159,8 +158,8 @@ struct tb2_layout {
     int group_cap[2];
     int num_groups[2];
     int* group_off[2];     // [G+1] scene indices, device
-    // round tables of sparse_layer1_pair (one per (layer width, unit count, CTAs per unit)), built on first use
-    struct PairPlan { int OUT, units_max, nC, units, rounds_per_unit, max_slots, R; void* dev; int* tile_slots; float* partials; };
+    // round tables of sparse_layer1_pair (one per (layer width, unit count)), built on first use
+    struct PairPlan { int OUT, units_max, units, rounds_per_unit; void* dev; };
     std::list<PairPlan> pair_plans;           // (list: entries are handed out by pointer)
     std::vector<void*> owned;
 };
@@ -220,9 +219,8 @@ int launch_pool_prepare(const tb2_lstm* m, const tb2_layout* l, const float* hid
                         const float* obs1, const float* obs2, int skip_masked, int write_pairs,
                         int write_emb, Workspace* ws, cudaStream_t st);
 // pooled_out fp32 and/or (pool_hi, pool_lo) bf16 split (either may be null, not both)
-// keep_hidden: the caller reads hidden1 afterwards (training recompute): the fused layer-1 + layer-2 kernel is not used
 int launch_pool_mlp(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float* pooled_out,
-                    void* pool_hi, void* pool_lo, cudaStream_t st, bool keep_hidden = false);
+                    void* pool_hi, void* pool_lo, cudaStream_t st);
 int launch_gates(const tb2_lstm* m, const tb2_layout* l, int phase, const float* obs1,
                  const float* obs2, const float* pooled, const float* h_in, const float* c_in,
                  float* h_out, float* c_out, float* normal_out, float* pos_out, cudaStream_t st);
@@ -232,12 +230,10 @@ int launch_repack_layer1_nat(const float* W1, void* hi, void* lo, int OUT, int c
 bool sparse_tc_supported(const tb2_lstm* m, const tb2_layout* l, int gsel);
 int launch_sparse_tc(const tb2_lstm* m, const tb2_layout* l, int gsel, Workspace* ws, float* out, void* out_hi,
                      void* out_lo, cudaStream_t st);
-// round-2 kernel of the same layer (pedestrians on the M side; mode 1 = one CTA, 2 = CTA pair with cta_group::2)
+// round-2 kernel of the same layer (pedestrians on the M side, CTA pair with cta_group::2)
 bool sparse_pair_supported(const tb2_lstm* m, const tb2_layout* l);
-int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, int mode, Workspace* ws, float* out, void* out_hi,
-                       void* out_lo, bool fuse2, cudaStream_t st);
-bool sparse_pair_can_fuse(const tb2_lstm* m);
-int launch_repack_layer2_sw(const float* W2, void* dst, int N2, int K, cudaStream_t st);
+int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float* out, void* out_hi, void* out_lo,
+                       cudaStream_t st);
 int launch_repack_layer1_sw(const float* W1, void* hi, void* lo, int OUT, int cells, cudaStream_t st);
 int launch_hidden_mlp_pool(const tb2_lstm* m, const tb2_layout* l, const float* hidden, const float* obs1,
                            const float* obs2, float* out, cudaStream_t st);

@@ -289,24 +289,6 @@ __global__ void add_bias_kernel(const float* __restrict__ a, const float* __rest
     if (i < n) out[i] = a[i] + b[i];
 }
 
-// pool.embedding.0.weight [d1][C * cells] (channel-major columns) -> bf16 (hi, lo) [d1][Kp] with columns in
-// (cell, channel) order, zero-padded to Kp: the B operand of the dense grid GEMM (occupancy / directional)
-__global__ void grid_weight_split_kernel(const float* __restrict__ W1, __nv_bfloat16* __restrict__ hi,
-                                         __nv_bfloat16* __restrict__ lo, int d1, int C, int cells, int Kp) {
-    const size_t total = (size_t)d1 * Kp;
-    for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
-        const int n = (int)(idx / Kp), k = (int)(idx - (size_t)n * Kp);
-        float v = 0.f;
-        if (k < C * cells) {
-            const int cell = k / C, c = k - cell * C;
-            v = W1[(size_t)n * C * cells + (size_t)c * cells + cell];
-        }
-        const __nv_bfloat16 h = __float2bfloat16_rn(v);
-        hi[idx] = h;
-        lo[idx] = __float2bfloat16_rn(v - __bfloat162float(h));
-    }
-}
-
 // outT[c][o] = sum_m Win[o][m] * w[m][c]   (E x E matrices; AttentionMLPPooling: in-projection after wq / wk / wv)
 __global__ void combine_proj_kernel(const float* __restrict__ Win, const float* __restrict__ w, float* __restrict__ outT, int E) {
     const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -473,21 +455,12 @@ int launch_repack(tb2_lstm* m, const tb2_lstm_weights* w, cudaStream_t st) {
         if (m->Wt1_sw_hi &&
             (rc = launch_repack_layer1_sw(w->pool_embedding_weight[0], m->Wt1_sw_hi, m->Wt1_sw_lo, m->mlp_dims[1], m->cells, st)))
             return rc;
-        if (m->W_hi[0]) {
-            const int k0p = (m->C * m->cells + 63) / 64 * 64;
-            grid_weight_split_kernel<<<256, 256, 0, st>>>(w->pool_embedding_weight[0], (__nv_bfloat16*)m->W_hi[0],
-                                                          (__nv_bfloat16*)m->W_lo[0], m->mlp_dims[1], m->C, m->cells, k0p);
-            TB2_LAUNCH_CHECK();
-        }
         for (int layer = 1; layer < m->n_mlp; ++layer) {
             TB2_REQUIRE(w->pool_embedding_weight[layer] && w->pool_embedding_bias[layer], "pool.embedding layer missing");
             transpose_kernel<<<512, 256, 0, st>>>(w->pool_embedding_weight[layer], m->WT[layer],
                                                   m->mlp_dims[layer + 1], m->mlp_dims[layer]);
             TB2_LAUNCH_CHECK();
             if ((rc = copy_dev(w->pool_embedding_bias[layer], m->bl[layer], (size_t)m->mlp_dims[layer + 1], st))) return rc;
-            if (layer == 1 && m->W2_sw &&
-                (rc = launch_repack_layer2_sw(w->pool_embedding_weight[1], m->W2_sw, m->mlp_dims[2], m->mlp_dims[1], st)))
-                return rc;
             if (m->W_hi[layer] &&
                 (rc = launch_split_bf16(w->pool_embedding_weight[layer], m->W_hi[layer], m->W_lo[layer],
                                         (size_t)m->mlp_dims[layer] * m->mlp_dims[layer + 1], st)))

@@ -13,6 +13,7 @@
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
+#include <cstring>
 #include <vector>
 
 #include "common.cuh"
@@ -1063,34 +1064,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) pool_rows_kernel(RowsParams p
     }
 }
 
-// Dense grid row of every pedestrian for the tcgen05 first Linear (occupancy / directional): [M][Kp] bf16 (hi, lo),
-// (value - constant) at the winners' (cell, channel) columns, zero elsewhere (the bias carries constant * sum W).
-// One warp per row.
-__global__ void __launch_bounds__(256) grid_rows_split_kernel(const int* __restrict__ win_count, const uint32_t* __restrict__ win_ent,
-                                                              const float* __restrict__ win_val, int M, int C, int nm1, int Kp,
-                                                              float constant, __nv_bfloat16* __restrict__ hi,
-                                                              __nv_bfloat16* __restrict__ lo) {
-    grid_dep_wait();
-    grid_dep_launch();
-    const int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-    if (row >= M) return;
-    uint4* h4 = reinterpret_cast<uint4*>(hi + (size_t)row * Kp);
-    uint4* l4 = reinterpret_cast<uint4*>(lo + (size_t)row * Kp);
-    for (int i = lane; i < Kp / 8; i += 32) { h4[i] = make_uint4(0u, 0u, 0u, 0u); l4[i] = make_uint4(0u, 0u, 0u, 0u); }
-    __syncwarp();
-    const int cnt = win_count[row];
-    for (int e = lane; e < cnt; e += 32) {
-        const uint32_t ent = win_ent[(size_t)row * nm1 + e];
-        const int cell = (int)(ent >> 16);
-        for (int c = 0; c < C; ++c) {
-            const float v = win_val[((size_t)row * nm1 + e) * 2 + c] - constant;
-            const __nv_bfloat16 h = __float2bfloat16_rn(v);
-            hi[(size_t)row * Kp + cell * C + c] = h;
-            lo[(size_t)row * Kp + cell * C + c] = __float2bfloat16_rn(v - __bfloat162float(h));
-        }
-    }
-}
-
 // returns the column chunk width the row kernel can use for this model (0 = does not fit)
 static int pool_rows_chunk(const tb2_lstm* m, int OUT) {
     if (m->cfg.pool_type == TB2_POOL_SOCIAL || m->C > 2) return 0;
@@ -1147,7 +1120,7 @@ static int launch_l1_t(const L1Params& p, int groups, size_t smem, cudaStream_t 
 
 // Grid -> pooled vector (GridBasedPooling.forward after the grid is known, :106-110).
 int launch_pool_mlp(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float* pooled_out,
-                    void* pool_hi, void* pool_lo, cudaStream_t st, bool keep_hidden) {
+                    void* pool_hi, void* pool_lo, cudaStream_t st) {
     const int nm1 = l->n_max > 1 ? l->n_max - 1 : 1;
     // producers that cannot write the bf16 split themselves go through fp32 scratch + split_rows
     const bool want_split = pool_hi != nullptr;
@@ -1203,50 +1176,22 @@ int launch_pool_mlp(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float
         p.out_lo = reinterpret_cast<__nv_bfloat16*>(pool_lo);
     }
     int rc;
-    const char* sp_env = getenv("TB2_SPARSE");       // debug knob: "mma" forces the warp-level MMA kernel,
-    const bool allow_tc = !(sp_env && sp_env[0] == 'm');     // "bucket" the per-cell bucket kernel, "tc" round 1's
-    const bool allow_rows = !(sp_env && sp_env[0] == 'b');   // tcgen05 kernel
-    int pair_mode = 3;                                       // default: the round-2 CTA-pair kernel with the A operand in tensor
-    if (sp_env && sp_env[0] == 'p') pair_mode = 2;           // memory; "pair": A in shared memory; "solo": one CTA per unit;
-    if (sp_env && sp_env[0] == 's' && sp_env[1] == 'o') pair_mode = 1;       // "tc" / "mma" / "bucket": the round-1 kernels
-    if (sp_env && (sp_env[0] == 't' || sp_env[0] == 'm' || sp_env[0] == 'b')) pair_mode = 0;
-    if (sp_env && sp_env[0] == 't' && sp_env[1] == 's') pair_mode = 3;
-    // TB2_GRID_TC=1 (opt-in): built and parity-green, but at the BASELINE batch two launches (grid rows 7-9 us + dense GEMM)
-    // only tie with pool_rows (17-21 us) in inference and cost the launch-bound D-LSTM training step 0.5 ms of host time
-    // (tensor-map encodes per call): profiles/round2_grid_tc_experiment.txt
-    const char* gtc = getenv("TB2_GRID_TC");
-    const int k0p = (m->C * m->cells + 63) / 64 * 64;
-    size_t wmax_floats = 1;
-    for (int i = 1; i <= m->n_mlp; ++i) wmax_floats = std::max(wmax_floats, (size_t)m->mlp_dims[i]);
-    if (!social && m->W_hi[0] != nullptr && gtc && gtc[0] == '1' && (size_t)k0p * 2 <= wmax_floats * sizeof(float) &&
-        m->n_mlp == 1) {     // deeper embeddings keep their layer-1 output in the same scratch
-        // occupancy / directional: explicit grid rows (bf16 hi | lo, in the activation scratch) -> dense 3-pass tcgen05 GEMM
-        __nv_bfloat16* a_hi = reinterpret_cast<__nv_bfloat16*>(ws->act[0]);
-        __nv_bfloat16* a_lo = reinterpret_cast<__nv_bfloat16*>(ws->act[1]);
-        {
-            KernelTimer kt("grid_rows_split", st);
-            launch_pdl(grid_rows_split_kernel, dim3((l->M + 7) / 8), dim3(256), 0, st, (const int*)ws->win_count,
-                       (const uint32_t*)ws->win_ent, (const float*)ws->win_val, l->M, m->C, nm1, k0p, m->cfg.constant, a_hi, a_lo);
-        }
-        TB2_LAUNCH_CHECK();
-        float* y = p.out;
-        if (y == nullptr && p.out_hi == nullptr) y = ws->pooled;
-        rc = launch_dense_tc(a_hi, a_lo, m->W_hi[0], m->W_lo[0], m->base1, y, p.out_hi, p.out_lo, l->M, k0p, d1, 1, st);
-    } else
-    if (allow_rows && pool_rows_chunk(m, d1) > 0) {   // occupancy / directional: weights resident in smem
+    // TB2_SPARSE (A/B and debug knob) forces round 1's kernels: "tc" and "bucket" skip the pair kernel, "mma" also
+    // sparse_layer1_tc, "bucket" also pool_rows
+    enum { kL1Default, kL1Tc, kL1Mma, kL1Bucket } force = kL1Default;
+    if (const char* e = getenv("TB2_SPARSE")) {
+        if (!strcmp(e, "tc")) force = kL1Tc;
+        else if (!strcmp(e, "mma")) force = kL1Mma;
+        else if (!strcmp(e, "bucket")) force = kL1Bucket;
+        else if (e[0]) { set_error("TB2_SPARSE must be tc, mma or bucket"); return TB2_ERR_INVALID; }
+    }
+    if (force != kL1Bucket && pool_rows_chunk(m, d1) > 0) {   // occupancy / directional: weights resident in smem
         rc = launch_pool_rows(m, l, ws, d1, nm1, p.out, p.out_hi, p.out_lo, st);
     } else
-    if (pair_mode && ws->cell_row && sparse_pair_supported(m, l)) {   // social, 16 latent channels: CTA-pair tcgen05 kernel
-        // TB2_FUSE2=1: also run the 1024 -> 256 Linear inside the kernel (hidden1 never leaves the SM).  Built, parity-
-        // green (2.9e-7 vs the separate layer) and measured: it LOSES 1.3 % per forward at the BASELINE shape and the
-        // per-piece partial sums make results depend on the batch decomposition -- off by default
-        // (profiles/round2_fuse2_experiment.txt).
-        const char* f2 = getenv("TB2_FUSE2");
-        if (!keep_hidden && sparse_pair_can_fuse(m) && f2 && f2[0] == '1')
-            return launch_sparse_pair(m, l, pair_mode, ws, pooled_out, pool_hi, pool_lo, true, st);
-        rc = launch_sparse_pair(m, l, pair_mode, ws, p.out, p.out_hi, p.out_lo, false, st);
+    if (force == kL1Default && ws->cell_row && sparse_pair_supported(m, l)) {   // social, 16 latent channels: CTA-pair tcgen05 kernel
+        rc = launch_sparse_pair(m, l, ws, p.out, p.out_hi, p.out_lo, st);
     } else
-    if (allow_tc && sparse_tc_supported(m, l, 0)) {  // social, 16 latent channels: tcgen05 path
+    if (force != kL1Mma && sparse_tc_supported(m, l, 0)) {  // social, 16 latent channels: tcgen05 path
         rc = launch_sparse_tc(m, l, 0, ws, p.out, p.out_hi, p.out_lo, st);
     } else
     if (m->Wt1_hi != nullptr) {      // social, 16 latent channels: warp-level tensor-core path

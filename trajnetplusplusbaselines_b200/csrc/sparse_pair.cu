@@ -9,18 +9,15 @@
 // side.  Per grid cell c one K = 16 product
 //     D[p, col] += L_c[p, 0:16] . W_c[col, 0:16]
 // where L_c[p, :] is the latent vector of p's winning neighbour in cell c, or zero.
-//   * kPair: two CTAs (one TPC) run tcgen05.mma.cta_group::2 with M = 256: each CTA owns 128
-//     pedestrians (its own A tiles) and HALF of the weight columns of the tile (B is shared by the
-//     pair), so every weight byte fetched from L2 serves 256 pedestrians and each SM's shared memory
-//     holds, and its tensor core reads, only half of B.  Per cell and CTA: 9 KB of weights written,
-//     14 KB read by the three passes, 8 KB of A written and 12 KB read = 43 KB against a 415-cycle
-//     tensor floor (81 % of the 128 B/clk port); round 1's kernel needed 70 KB for 480 cycles.
-//   * A tiles (L_c, bf16 hi and lo, SWIZZLE_32B K-major) are written by four builder warps, one
-//     thread per pedestrian row, every row every cell (no re-zeroing, no buckets): the thread reads
-//     "which neighbour of mine sits in cell c" from the per-row cell map pool_prepare leaves in
-//     global memory (16 cells per 16-byte load, prefetched) and copies the neighbour's split latent
-//     vector from a per-tile table in shared memory.  (With the A operand in tensor memory instead,
-//     the 8 KB of tcgen05.st per cell were the bottleneck: profiles/round2_ts_experiment.txt.)
+//   * Two CTAs (one TPC) run tcgen05.mma.cta_group::2 with M = 256: each CTA owns 128 pedestrians (its own
+//     A operand) and HALF of the weight columns of the tile (B is shared by the pair), so every weight byte
+//     fetched from L2 serves 256 pedestrians and each SM's shared memory holds only half of B.
+//   * The A operand lives in tensor memory, in a ring of stages behind the accumulators.  Builder warps, one
+//     thread per pedestrian row (= TMEM lane), write every row of every cell (no re-zeroing, no buckets): the
+//     thread reads "which neighbour of mine sits in cell c" from the per-row cell map pool_prepare leaves in
+//     global memory (16 cells per 16-byte load, prefetched), copies the neighbour's split latent vector from a
+//     per-tile table in shared memory and stores it with one tcgen05.st per cell.  Shared memory carries only
+//     the weights, which buys a deep weight ring.
 //   * The weight slabs W_c are stored pre-swizzled (SWIZZLE_32B image) in global memory, so one
 //     plain bulk copy (cp.async.bulk) of any multiple of 16 rows lands the tile the UMMA
 //     descriptor expects.
@@ -29,14 +26,16 @@
 //     contexts (tile, column range) with at most 288 accumulator columns, so a range that straddles a
 //     tile boundary still keeps all SMs equally loaded (5120 pedestrians x 1024 columns on 74 pairs:
 //     8.65 blocks each, against 128 of 148 SMs busy in round 1).
-//   * Pipeline item = 4 grid cells (K = 64; 2 when a round spans two pedestrian tiles), 3 items in
-//     flight: one barrier round trip builders -> MMA issuers -> tcgen05.commit per item.
+//   * Pipeline item = 4 grid cells (K = 64) of the round's tile, or of both tiles of a two-tile round (2 cells
+//     when the round has more than 256 accumulator columns): one barrier round trip builders -> MMA issuers ->
+//     tcgen05.commit per item.
 //   * Precision: 3-pass bf16 (hi, lo) split, fp32 accumulation in TMEM, like the other kernels;
 //     results are bit-identical to sparse_layer1_tc_kernel (same products, same order per column).
+//   Measurements and the designs this one replaced: DESIGN.md section 4.1.
 //
-// Warp roles (512 threads): 0 = weight producer, 1 / 2 = MMA issuers of context 0 / 1 (leader CTA
-// only; 1 also owns the TMEM allocation), 4..7 = builders of A slot 0, 8..11 = builders of A slot 1
-// (second pedestrian tile of a round); warps 4..15 run the epilogue (3 per TMEM lane quarter).
+// Warp roles (512 threads): 0 = weight producer, 1 / 2 = MMA issuers (leader CTA only; 1 also owns the TMEM
+// allocation), 3 = weight relay, 4..7 / 8..11 = builders (one-tile round: even / odd items; two-tile round:
+// one tile each); all 16 warps run the epilogue (4 per TMEM lane quarter).
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cstdio>
@@ -52,38 +51,24 @@ namespace tb2 {
 constexpr int kSpThreads = 512;
 constexpr int kSpSA = 3;                 // ring of A stages (built on the fly, short turn-around)
 constexpr int kSpSBMax = 8;              // ring of weight stages (bulk copies from L2: ~1500 cycles from request to landing):
-                                         // 3 x 4 cells (one tile) / 5 x 2 cells (two tiles); TS variant, whose A ring
-                                         // lives in tensor memory: 5 x 4 cells / 8 x 2 cells over the freed shared memory
+                                         // 5 x 4 cells (one tile) / 8 x 2 cells (two tiles)
 constexpr int kSpMaxBlocks = 9;          // 32-column blocks per round (288 accumulator columns)
 constexpr int kSpDCols = kSpMaxBlocks * 32;
 constexpr int kSpMaxCells = 256;
 constexpr int kSpLatRows = 256;          // local latent table (rows of the scenes a 128-row tile touches) + 1
-constexpr uint32_t kSpATile = 128 * 32;  // one A tile: 128 pedestrian rows x 16 k bf16
-// Pipeline item: one-tile round = 4 grid cells (K = 64) of the tile; two-tile round = 2 cells of BOTH tiles (the
-// two accumulator chains are interleaved MMA by MMA).  Either way an A stage is 4 x (hi | lo) tiles = 32 KB and
-// the weights of an item are at most 4 x 9 KB (one tile: 3 stages) or 2 x 9 KB (two tiles: 5 stages).
-constexpr uint32_t kSpAStage = 4u * 2u * kSpATile;
 constexpr uint32_t kSpBCell = (uint32_t)(kSpDCols / 2) * 64u;          // bytes of weights per cell and CTA of a pair (288 columns)
-constexpr uint32_t kSpBRing = 3u * 4u * kSpBCell;
-// dynamic shared memory behind the 1024-byte alignment: [A ring | weight ring | latent table 0]; the second
-// latent table of a two-tile round sits in the unused tail of the weight ring (5 x 2 cells < 3 x 4 cells)
-constexpr size_t kSpDynBytes = (size_t)kSpSA * kSpAStage + kSpBRing + (size_t)kSpLatRows * 64;
-static_assert((size_t)5 * 2 * kSpBCell + (size_t)kSpLatRows * 64 <= kSpBRing, "two-tile rounds: second latent table");
-static_assert((size_t)5 * 4 * kSpBCell <= kSpDynBytes - (size_t)kSpLatRows * 64, "TS: one-tile weight ring");
-static_assert((size_t)8 * 2 * kSpBCell <= kSpDynBytes - (size_t)2 * kSpLatRows * 64, "TS: two-tile weight ring");
+// dynamic shared memory behind the 1024-byte alignment: [weight ring | latent table 1 | latent table 0] (the second
+// latent table is the one of a two-tile round)
+constexpr size_t kSpDynBytes = 220 * 1024;
+static_assert((size_t)5 * 4 * kSpBCell <= kSpDynBytes - (size_t)kSpLatRows * 64, "one-tile weight ring");
+static_assert((size_t)8 * 2 * kSpBCell <= kSpDynBytes - (size_t)2 * kSpLatRows * 64, "two-tile weight ring");
 static_assert(1024 + kSpDynBytes + 64 <= 227 * 1024 - 1024, "shared memory budget");
-// fused layer-2 tail: hidden1 of the round as A tiles (one (hi | lo) tile pair per 16 columns) + a ring of W2 k-step tiles
-constexpr int kSpN2 = 256;
-constexpr int kSpTailStages = 6;
-constexpr uint32_t kSpA2Bytes = (uint32_t)(kSpDCols / 16) * 2u * kSpATile;
-static_assert(kSpA2Bytes + 4u * (uint32_t)kSpN2 * 64u <= kSpDynBytes, "tail: one CTA per unit, 4 stages");
-static_assert(kSpA2Bytes + (uint32_t)kSpTailStages * (uint32_t)(kSpN2 / 2) * 64u <= kSpDynBytes, "tail: pair, 6 stages");
 
-// TS variant (A operand in tensor memory): accumulators in TMEM columns [0, 288), the A ring behind them: 3 stages x
-// 64 columns (one-tile item: 4 cells x (hi 8 | lo 8) columns; two-tile item: 2 cells x 2 tiles x 16 columns)
-constexpr uint32_t kSpTsACol0 = 320;
-constexpr uint32_t kSpTsAStageCols = 64;
-static_assert(kSpDCols <= (int)kSpTsACol0 && kSpTsACol0 + kSpSA * kSpTsAStageCols <= 512, "TMEM budget of the TS variant");
+// TMEM: accumulators in columns [0, 288), the A ring behind them: 3 stages x 64 columns (one-tile item: 4 cells x
+// (hi 8 | lo 8) columns; two-tile item of 2 cells: 2 cells x 2 tiles x 16 columns)
+constexpr uint32_t kSpACol0 = 320;
+constexpr uint32_t kSpAStageCols = 64;
+static_assert(kSpDCols <= (int)kSpACol0 && kSpACol0 + kSpSA * kSpAStageCols <= 512, "TMEM budget");
 
 __device__ __forceinline__ uint32_t sp_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void sp_mbar_init(uint32_t bar, uint32_t count) {
@@ -95,7 +80,7 @@ __device__ __forceinline__ void sp_mbar_expect_tx(uint32_t bar, uint32_t bytes) 
 // arrive on a barrier of the leader CTA (cluster address).  Default semantics (.release.cta) like CUTLASS'
 // ClusterBarrier::arrive: a .release.cluster arrive per builder warp and item cost ~2000 cycles of serial
 // latency per item (measured), and the data this signal publishes is read by THIS SM's tensor core, behind
-// the fence.proxy.async each builder thread executed.
+// the tcgen05.fence each builder thread executed.
 __device__ __forceinline__ void sp_mbar_arrive_cluster(uint32_t cluster_addr) {
     asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
@@ -126,33 +111,17 @@ __device__ __forceinline__ void sp_bulk_load(uint32_t dst, const void* src, uint
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
 }
-// completion of all earlier tcgen05.mma of this thread -> arrive on `bar` (pair: in both CTAs)
-template <bool kPair>
+// completion of all earlier tcgen05.mma of this thread -> arrive on `bar` in both CTAs of the pair
 __device__ __forceinline__ void sp_commit(uint32_t bar) {
-    if (kPair) {
-        const uint16_t mask = 3;
-        asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                     ::"r"(bar), "h"(mask) : "memory");
-    } else {
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-    }
-}
-__device__ __forceinline__ void sp_tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-          "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]),
-          "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]),
-          "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-        : "r"(taddr));
+    const uint16_t mask = 3;
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                 ::"r"(bar), "h"(mask) : "memory");
 }
 
 
 // One round of a unit: `n0` 32-column blocks of pedestrian tile `tile` starting at block `blk0`, then (n1 > 0) the
 // first `n1` blocks of tile + 1.  Planned on the host (plan_rounds) so that no piece is narrower than 3 blocks.
-struct SpRound { int tile, blk0, n0, n1, slot0, slot1; };      // slot: index of the piece among the pieces of its tile (fused layer 2)
+struct SpRound { int tile, blk0, n0, n1; };
 
 __device__ __forceinline__ void sp_tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     asm volatile(
@@ -175,52 +144,20 @@ struct SpParams {
     __nv_bfloat16* out_hi;           // bf16 split [M, OUT] or null
     __nv_bfloat16* out_lo;
     const SpRound* rounds;           // [units * rounds_per_unit] (plan_rounds)
-    // fused second Linear (two_layer, 256 outputs): hidden1 stays on chip; every piece writes its K-slice partial sums
-    const unsigned char* w2;         // bf16 [OUT / 16][N2 / 8][hi: 8 rows x 16 | lo: 8 rows x 16] of pool.embedding.2.weight, or null
-    float* partials;                 // [tiles][max_slots][R][N2] fp32
-    int N2, max_slots;
     int M, OUT, cells, rounds_per_unit;
     float constant;
-    long long* dbg;                  // optional [units * nC, 8] cycle counters (TB2_L1_DEBUG=1)
+    long long* dbg;                  // optional [2 * units, 8] cycle counters (TB2_L1_DEBUG=1)
 };
 
-// SS-form MMA with 64-bit shared-memory descriptors kept in registers (the issuing thread is a single
-// thread: every instruction between two MMAs counts)
-template <bool kPair>
-__device__ __forceinline__ void sp_umma(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    if (kPair)
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-    else
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-
-// TS form: A = 128 lanes x 8 TMEM columns (16 bf16 of K per lane) of each CTA, B from shared memory
-template <bool kPair>
+// MMA with A = 128 lanes x 8 TMEM columns (16 bf16 of K per lane) of each CTA, B from shared memory (64-bit
+// descriptor kept in registers: the issuing thread is a single thread, every instruction between two MMAs counts)
 __device__ __forceinline__ void sp_umma_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-    if (kPair)
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-    else
-        asm volatile(
-            "{\n"
-            ".reg .pred p;\n"
-            "setp.ne.b32 p, %4, 0;\n"
-            "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n"
-            "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n"
+        "}\n" ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
 }
 // one pedestrian row (lane) of one cell: hi (8 columns) | lo (8 columns)
 __device__ __forceinline__ void sp_tmem_st16(uint32_t taddr, const uint4& h0, const uint4& h1, const uint4& l0, const uint4& l1) {
@@ -229,36 +166,11 @@ __device__ __forceinline__ void sp_tmem_st16(uint32_t taddr, const uint4& h0, co
                    "r"(l0.x), "r"(l0.y), "r"(l0.z), "r"(l0.w), "r"(l1.x), "r"(l1.y), "r"(l1.z), "r"(l1.w) : "memory");
 }
 
-// byte offset of (row r, 16-byte chunk c) inside a SWIZZLE_32B K-major tile
-__device__ __forceinline__ uint32_t sp_sw32(uint32_t r, uint32_t c) { return r * 32u + ((c ^ ((r >> 2) & 1u)) << 4); }
-
-// Builder body for one pipeline item of KC cells; `bytes` holds the KC cell-map bytes of this row (LSB first).
+// Builder body for one pipeline item of KC cells: the row's (hi | lo) vectors of the item's cells go to the lane's
+// 16 TMEM columns per cell; `bytes` holds the KC cell-map bytes of this row (LSB first).
 template <int KC>
-__device__ __forceinline__ void sp_build_item(unsigned char* a_item, uint32_t a_stride, uint32_t bytes, int kcn, uint32_t r,
-                                              int off_r, int nlat, const uint4* lh, const uint4* ll) {
-#pragma unroll
-    for (int kc = 0; kc < KC; ++kc) {
-        if (kc < kcn) {
-            const uint32_t j = (bytes >> (8 * kc)) & 0xffu;
-            uint4 h0 = make_uint4(0u, 0u, 0u, 0u), h1 = h0, l0 = h0, l1 = h0;
-            if (j != 0xffu) {
-                const int li = j == 0xfeu ? nlat : (int)j + off_r;
-                h0 = lh[li * 2]; h1 = lh[li * 2 + 1];
-                l0 = ll[li * 2]; l1 = ll[li * 2 + 1];
-            }
-            unsigned char* t = a_item + (size_t)kc * a_stride;
-            *reinterpret_cast<uint4*>(t + sp_sw32(r, 0)) = h0;
-            *reinterpret_cast<uint4*>(t + sp_sw32(r, 1)) = h1;
-            *reinterpret_cast<uint4*>(t + kSpATile + sp_sw32(r, 0)) = l0;
-            *reinterpret_cast<uint4*>(t + kSpATile + sp_sw32(r, 1)) = l1;
-        }
-    }
-}
-
-// TS variant: the row's (hi | lo) vectors of the item's cells go to the lane's 16 TMEM columns per cell
-template <int KC>
-__device__ __forceinline__ void sp_build_item_ts(uint32_t a_item, uint32_t cell_cols, uint32_t bytes, int off_r, int nlat,
-                                                 const uint4* lh, const uint4* ll) {
+__device__ __forceinline__ void sp_build_item(uint32_t a_item, uint32_t cell_cols, uint32_t bytes, int off_r, int nlat,
+                                              const uint4* lh, const uint4* ll) {
 #pragma unroll
     for (int kc = 0; kc < KC; ++kc) {
         const uint32_t j = (bytes >> (8 * kc)) & 0xffu;
@@ -272,18 +184,18 @@ __device__ __forceinline__ void sp_build_item_ts(uint32_t a_item, uint32_t cell_
     }
 }
 
-// Builder role of one warp for one round: thread = pedestrian row r; `cr` = the row's cell map (16 cells per
-// uint4) or null for rows past the end.  One-tile round: the two builder groups (warps 4..7 / 8..11) take the even
-// / odd items.  Two-tile round (kTwo): group bg builds the tiles of pedestrian tile bg inside EVERY item.
-template <int KC, bool kTwo, bool kTS>
-__device__ __forceinline__ void sp_builder(const uint4* cr, int groups, unsigned char* a_ring, uint32_t a_tmem, int bg,
-                                           uint32_t r, int off_r, int nlat, const uint4* lh, const uint4* ll,
-                                           uint64_t* empty_a, const uint32_t (&full_remote)[kSpSA], int lane, long long& wait_e,
-                                           uint32_t SA = kSpSA, uint32_t ts_stage_cols = kSpTsAStageCols) {
+// Builder role of one warp for one round: thread = pedestrian row; `cr` = the row's cell map (16 cells per uint4) or
+// null for rows past the end.  One-tile round: the two builder groups (warps 4..7 / 8..11) take the even / odd items
+// (KC = 4).  Two-tile round (kTwo): group bg builds the A operand of pedestrian tile bg inside EVERY item.
+template <int KC, bool kTwo>
+__device__ __forceinline__ void sp_builder(const uint4* cr, int groups, uint32_t a_tmem, int bg, int off_r, int nlat,
+                                           const uint4* lh, const uint4* ll, uint64_t* empty_a,
+                                           const uint32_t (&full_remote)[kSpSA], int lane, long long& wait_e,
+                                           uint32_t SA, uint32_t stage_cols) {
+    static_assert(kTwo || KC == 4, "one-tile rounds use 4-cell items");
     const uint4 none = make_uint4(~0u, ~0u, ~0u, ~0u);
     constexpr int ipg = 16 / KC;                       // items per 16-cell load of the row's cell map
     constexpr int step = kTwo ? 1 : 2;
-    constexpr uint32_t a_stride = kTwo ? 4u * kSpATile : 2u * kSpATile;       // bytes between the cells of an item
     uint4 cur = cr ? __ldg(cr) : none;
     for (int g16 = 0; g16 < groups; ++g16) {
         const uint4 next = (cr && g16 + 1 < groups) ? __ldg(cr + g16 + 1) : none;     // prefetched one group ahead
@@ -297,23 +209,16 @@ __device__ __forceinline__ void sp_builder(const uint4* cr, int groups, unsigned
                 bytes = KC == 4 ? w : (w >> (8 * (c & 3))) & ((1u << (8 * (KC & 3))) - 1u);
             } else {
                 g = (uint32_t)(g16 * ipg + 2 * jj + bg);
-                if (KC == 4) bytes = jj == 0 ? (bg ? cur.y : cur.x) : (bg ? cur.w : cur.z);
-                else bytes = ((jj == 0 ? cur.x : jj == 1 ? cur.y : jj == 2 ? cur.z : cur.w) >> (16 * bg)) & 0xffffu;
+                bytes = jj == 0 ? (bg ? cur.y : cur.x) : (bg ? cur.w : cur.z);
             }
             const uint32_t sa = g % SA, pa = (g / SA) & 1u;
             const long long tw0 = clock64();
             sp_mbar_wait(sp_smem_u32(&empty_a[sa]), pa ^ 1u);
             wait_e += clock64() - tw0;
-            if (kTS) {
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                sp_build_item_ts<KC>(a_tmem + sa * ts_stage_cols, kTwo ? 32u : 16u, bytes, off_r, nlat, lh, ll);
-                asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
-            } else {
-                sp_build_item<KC>(a_ring + (size_t)sa * kSpAStage, a_stride, bytes, KC, r, off_r, nlat, lh, ll);
-                // generic-proxy writes of the tiles -> visible to the tensor core's async-proxy reads
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            }
-            if (kTS) asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+            sp_build_item<KC>(a_tmem + sa * stage_cols, kTwo ? 32u : 16u, bytes, off_r, nlat, lh, ll);
+            asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
             if (lane == 0) sp_mbar_arrive_cluster(full_remote[sa]);
         }
@@ -321,31 +226,25 @@ __device__ __forceinline__ void sp_builder(const uint4* cr, int groups, unsigned
     }
 }
 
-template <bool kPair, bool kTS>
 __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpParams p) {
-    constexpr int nC = kPair ? 2 : 1;
+    constexpr int R = 256;                                // pedestrian rows per tile: 128 per CTA of the pair
     extern __shared__ __align__(1024) unsigned char smem_sp[];
-    __shared__ __align__(8) uint64_t full_a[kSpSA];       // leader: A tiles (both CTAs) built AND weights (both CTAs) landed
+    __shared__ __align__(8) uint64_t full_a[kSpSA];       // leader: A (both CTAs) built AND weights (both CTAs) landed
     __shared__ __align__(8) uint64_t empty_a[kSpSA];      // MMAs that read the A stage done
     __shared__ __align__(8) uint64_t full_b[kSpSBMax];    // local weight slabs landed
     __shared__ __align__(8) uint64_t empty_b[kSpSBMax];   // MMAs that read the weight stage done
     __shared__ __align__(8) uint64_t acc_full_bar;
-    __shared__ __align__(8) uint64_t full_w[kSpTailStages];      // tail: W2 k-step tile landed (local)
-    __shared__ __align__(8) uint64_t empty_w[kSpTailStages];     // tail: MMAs that read the stage done
-    __shared__ __align__(8) uint64_t peer_w[kSpTailStages];      // tail, leader: the peer CTA's tile landed
-    __shared__ __align__(8) uint64_t acc2_full_bar;
     __shared__ uint32_t tmem_base_slot;
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    uint32_t rank = 0;
-    if (kPair) asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
-    const int unit = kPair ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
+    uint32_t rank;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    const int unit = (int)(blockIdx.x >> 1);
     long long* dbg = p.dbg ? p.dbg + (size_t)blockIdx.x * 8 : nullptr;
     const long long t_begin = clock64();
 
-    const uint32_t ring = (sp_smem_u32(smem_sp) + 1023u) & ~1023u;          // A ring
+    const uint32_t ring = (sp_smem_u32(smem_sp) + 1023u) & ~1023u;          // weight ring
     unsigned char* ring_ptr = smem_sp + (ring - sp_smem_u32(smem_sp));
-    const uint32_t bring = kTS ? ring : ring + (uint32_t)kSpSA * kSpAStage;   // weight ring (TS: no A ring in shared memory)
     uint4* latH[2];
     uint4* latL[2];
     latH[0] = reinterpret_cast<uint4*>(ring_ptr + kSpDynBytes - (size_t)kSpLatRows * 64);
@@ -356,15 +255,9 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
     // ---- prologue: TMEM (the barriers are initialised per round) ----------------------------------
     if (warp == 1) {
         uint32_t ncols = 512;
-        if (kPair) {
-            asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-                         ::"r"(sp_smem_u32(&tmem_base_slot)), "r"(ncols) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-        } else {
-            asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                         ::"r"(sp_smem_u32(&tmem_base_slot)), "r"(ncols) : "memory");
-            asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-        }
+        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
+                     ::"r"(sp_smem_u32(&tmem_base_slot)), "r"(ncols) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
@@ -378,28 +271,26 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
 #pragma unroll
     for (int s = 0; s < kSpSA; ++s) {
         uint32_t local = sp_smem_u32(&full_a[s]);
-        if (kPair) asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(full_remote[s]) : "r"(local), "r"(0));
-        else full_remote[s] = local;
+        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(full_remote[s]) : "r"(local), "r"(0));
     }
 
-    const int R = 128 * nC;                               // pedestrian rows per tile
     uint32_t round_idx = 0;
     long long t_setup_sum = 0, t_loop_sum = 0, t_epi_sum = 0, wait_full = 0, wait_b = 0, wait_e = 0;
-    SpRound rd = {0, 0, 0, 0, 0, 0};
+    SpRound rd = {0, 0, 0, 0};
     for (int ri = 0; ri < p.rounds_per_unit; ++ri) {
         rd = p.rounds[(size_t)unit * p.rounds_per_unit + ri];
         if (rd.n0 == 0) continue;                         // padding round (uniform for the whole cluster)
         const long long t_r0 = clock64();
         const int nsub = rd.n1 > 0 ? 2 : 1;
         // pipeline shape of the round (the barriers are re-initialised for it)
-        // TS variant, two-tile round of <= 256 accumulator columns: items of 4 cells of both tiles (one barrier round trip per
+        // two-tile round of <= 256 accumulator columns: items of 4 cells of both tiles (one barrier round trip per
         // 4 cells instead of 2: the issuers of a two-tile round barely run ahead of the tensor pipe), 2 A stages of 128 TMEM
         // columns at [256, 512)
-        const bool wide_items = kTS && kPair && nsub == 2 && (rd.n0 + rd.n1) * 32 <= 256;
+        const bool wide_items = nsub == 2 && (rd.n0 + rd.n1) * 32 <= 256;
         const uint32_t SA = wide_items ? 2u : (uint32_t)kSpSA;
-        const uint32_t a_col0 = wide_items ? 256u : kSpTsACol0, a_stage_cols = wide_items ? 128u : kSpTsAStageCols;
-        const int KC = nsub == 2 ? (kPair ? (wide_items ? 4 : 2) : 1) : (kPair ? 4 : 2);     // grid cells per pipeline item
-        const uint32_t SB = nsub == 2 ? (wide_items ? 5u : (kTS ? 8u : 5u)) : (kTS ? 5u : 3u);   // weight stages
+        const uint32_t a_col0 = wide_items ? 256u : kSpACol0, a_stage_cols = wide_items ? 128u : kSpAStageCols;
+        const int KC = nsub == 2 && !wide_items ? 2 : 4;     // grid cells per pipeline item
+        const uint32_t SB = nsub == 2 && !wide_items ? 8u : 5u;   // weight stages
         const int n_items = p.cells / KC;                    // cells is a multiple of 16
         const uint32_t n_issuers = 2u;
         if (tid == 0) {
@@ -409,7 +300,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                     asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&empty_a[s2])) : "memory");
                 }
                 // builders per item and CTA: one group of 4 warps (one tile) or both groups (two tiles)
-                sp_mbar_init(sp_smem_u32(&full_a[s2]), ((nsub == 2 ? 8 : 4) + 1) * nC);        // + the weight relay
+                sp_mbar_init(sp_smem_u32(&full_a[s2]), ((nsub == 2 ? 8 : 4) + 1) * 2);        // + the weight relay
                 sp_mbar_init(sp_smem_u32(&empty_a[s2]), n_issuers);      // one tcgen05.commit per active MMA issuer
             }
             for (int s2 = 0; s2 < kSpSBMax; ++s2) {
@@ -422,32 +313,20 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             }
             if (round_idx > 0) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&acc_full_bar)) : "memory");
             sp_mbar_init(sp_smem_u32(&acc_full_bar), n_issuers);
-            for (int s2 = 0; s2 < kSpTailStages; ++s2) {
-                if (round_idx > 0) {
-                    asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&full_w[s2])) : "memory");
-                    asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&empty_w[s2])) : "memory");
-                    asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&peer_w[s2])) : "memory");
-                }
-                sp_mbar_init(sp_smem_u32(&full_w[s2]), 1);
-                sp_mbar_init(sp_smem_u32(&empty_w[s2]), 1);
-                sp_mbar_init(sp_smem_u32(&peer_w[s2]), 1);
-            }
-            if (round_idx > 0) asm volatile("mbarrier.inval.shared::cta.b64 [%0];" ::"r"(sp_smem_u32(&acc2_full_bar)) : "memory");
-            sp_mbar_init(sp_smem_u32(&acc2_full_bar), 1);
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         }
         // piece x: columns [col0[x], col0[x] + ncols[x]) of tile[x]; accumulators of piece 1 behind those of piece 0
         const int tile[2] = {rd.tile, rd.tile + 1};
         const int col0[2] = {rd.blk0 * 32, 0};
         const uint32_t ncols[2] = {(uint32_t)rd.n0 * 32u, (uint32_t)rd.n1 * 32u};
-        const uint32_t nr[2] = {ncols[0] / nC, ncols[1] / nC};              // rows of each piece's slab held by this CTA
+        const uint32_t nr[2] = {ncols[0] / 2, ncols[1] / 2};                // rows of each piece's slab held by this CTA
         const uint32_t b_cell = 64u * (nr[0] + nr[1]);                       // weight bytes per cell: piece 0 rows | piece 1 rows
         const uint32_t b_stage = (uint32_t)KC * b_cell;
         // weights of item `it` of this round -> stage it % SB (the producer thread; the stage must be free)
         auto load_item = [&](int it) {
             const uint32_t sb = (uint32_t)it % SB;
             const uint32_t bar = sp_smem_u32(&full_b[sb]);
-            const uint32_t st = bring + sb * b_stage;
+            const uint32_t st = ring + sb * b_stage;
             sp_mbar_expect_tx(bar, b_stage);
             for (int kc = 0; kc < KC; ++kc) {
                 const size_t cellsrc = (size_t)(it * KC + kc) * p.OUT;
@@ -499,14 +378,13 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             }
         }
         __syncthreads();
-        if (kPair) {      // the peer's barriers must be initialised before the first remote arrive / multicast commit
-            asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-            asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-        }
+        // the peer's barriers must be initialised before the first remote arrive / multicast commit
+        asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+        asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
         const long long t_r1 = clock64();
         t_setup_sum += t_r1 - (round_idx == 0 ? t_start : t_r0);
 
-        // MMA groups of a one-tile round: a 9-block piece is issued as N = 160 + 128 over the same A tiles
+        // MMA groups of a one-tile round: a 9-block piece is issued as N = 160 + 128 over the same A operand
         const bool split = ncols[0] > 256u;
 
         if (warp == 0) {
@@ -528,30 +406,24 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             // DIFFERENT items did not interleave, 800 cycles per cell instead of 432.) =====
             if (lane == 0 && rank == 0) {
                 const int gq = warp - 1;
-                const uint32_t a_desc_hi = (uint32_t)(256 >> 4) | (1u << 14) | (6u << 29);    // SBO 256 | version 1 | SWIZZLE_32B
                 const uint32_t b_desc_hi = (uint32_t)(512 >> 4) | (1u << 14) | (6u << 29);    // row groups alternate hi / lo
-                const uint64_t a_base = ((uint64_t)a_desc_hi << 32) | (uint64_t)((ring & 0x3FFFFu) >> 4);
-                const uint64_t b_base = ((uint64_t)b_desc_hi << 32) | (uint64_t)((bring & 0x3FFFFu) >> 4);
+                const uint64_t b_base = ((uint64_t)b_desc_hi << 32) | (uint64_t)((ring & 0x3FFFFu) >> 4);
                 const uint64_t bcell16 = b_cell >> 4;
                 const uint32_t idesc_base = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(R >> 4) << 24);
                 // MMA group of this issuer.  One tile: a 9-block piece is issued as N = 160 + 128 over the same A
-                // tiles by the two issuers, anything narrower by issuer 0 alone.  Two tiles: issuer gq owns piece gq
-                // (its own A tiles inside the stage).  Both issuers wake on the same barrier and issue the same
+                // operand by the two issuers, anything narrower by issuer 0 alone.  Two tiles: issuer gq owns piece gq
+                // (its own A columns inside the stage).  Both issuers wake on the same barrier and issue the same
                 // number of MMAs per item, so their two accumulator chains interleave in the tensor core's queue.
                 uint32_t gn, d;
-                uint64_t a_off16, a_cell16, b_off16;
+                uint64_t b_off16;
                 if (nsub == 2) {
                     gn = ncols[gq];
                     d = tmem_base + (gq ? ncols[0] : 0u);
-                    a_off16 = (uint64_t)((uint32_t)gq * 2u * kSpATile >> 4);
-                    a_cell16 = (4u * kSpATile) >> 4;
                     b_off16 = gq ? (uint64_t)(nr[0] * 4u) : 0u;                      // piece 1's rows behind piece 0's
                 } else {
                     gn = split ? (gq == 0 ? 160u : ncols[0] - 160u) : (gq == 0 ? ncols[0] : 0u);
                     d = tmem_base + ((split && gq == 1) ? 160u : 0u);
-                    a_off16 = 0u;
-                    a_cell16 = (2u * kSpATile) >> 4;
-                    b_off16 = (split && gq == 1) ? (uint64_t)((160u / nC) * 4u) : 0u;   // the group's rows inside a cell
+                    b_off16 = (split && gq == 1) ? (uint64_t)((160u / 2) * 4u) : 0u;    // the group's rows inside a cell
                 }
                 const bool have = gn > 0;
                 const uint32_t idesc = idesc_base | ((gn >> 3) << 17);
@@ -562,40 +434,26 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                     sp_mbar_wait_cluster(sp_smem_u32(&full_a[sa]), pa);
                     wait_full += clock64() - t0;
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                    if (have && kTS) {
+                    if (have) {
                         // A from tensor memory: stage sa, (two tiles: the issuer's own tile inside every cell)
                         uint32_t at = tmem_base + a_col0 + sa * a_stage_cols + (nsub == 2 ? (uint32_t)gq * 16u : 0u);
                         const uint32_t at_cell = nsub == 2 ? 32u : 16u;
                         uint64_t bd = b_base + (uint64_t)(sb * (b_stage >> 4)) + b_off16;
-                        sp_umma_ts<kPair>(d, at, bd, idesc, it > 0 ? 1u : 0u);                  // hi . hi
-                        sp_umma_ts<kPair>(d, at + 8u, bd, idesc, 1u);                           // lo . hi
-                        sp_umma_ts<kPair>(d, at, bd + (256u >> 4), idesc, 1u);                  // hi . lo
+                        sp_umma_ts(d, at, bd, idesc, it > 0 ? 1u : 0u);                  // hi . hi
+                        sp_umma_ts(d, at + 8u, bd, idesc, 1u);                           // lo . hi
+                        sp_umma_ts(d, at, bd + (256u >> 4), idesc, 1u);                  // hi . lo
 #pragma unroll 3
                         for (int kc = 1; kc < KC; ++kc) {
                             at += at_cell; bd += bcell16;
-                            sp_umma_ts<kPair>(d, at, bd, idesc, 1u);
-                            sp_umma_ts<kPair>(d, at + 8u, bd, idesc, 1u);
-                            sp_umma_ts<kPair>(d, at, bd + (256u >> 4), idesc, 1u);
-                        }
-                    } else if (have) {
-                        // the start-address field never carries into the next field (addresses < 256 KB)
-                        uint64_t ad = a_base + (uint64_t)(sa * (kSpAStage >> 4)) + a_off16;
-                        uint64_t bd = b_base + (uint64_t)(sb * (b_stage >> 4)) + b_off16;
-                        sp_umma<kPair>(d, ad, bd, idesc, it > 0 ? 1u : 0u);                     // hi . hi
-                        sp_umma<kPair>(d, ad + (kSpATile >> 4), bd, idesc, 1u);                 // lo . hi
-                        sp_umma<kPair>(d, ad, bd + (256u >> 4), idesc, 1u);                     // hi . lo
-#pragma unroll 3
-                        for (int kc = 1; kc < KC; ++kc) {
-                            ad += a_cell16; bd += bcell16;
-                            sp_umma<kPair>(d, ad, bd, idesc, 1u);
-                            sp_umma<kPair>(d, ad + (kSpATile >> 4), bd, idesc, 1u);
-                            sp_umma<kPair>(d, ad, bd + (256u >> 4), idesc, 1u);
+                            sp_umma_ts(d, at, bd, idesc, 1u);
+                            sp_umma_ts(d, at + 8u, bd, idesc, 1u);
+                            sp_umma_ts(d, at, bd + (256u >> 4), idesc, 1u);
                         }
                     }
-                    sp_commit<kPair>(sp_smem_u32(&empty_a[sa]));
-                    sp_commit<kPair>(sp_smem_u32(&empty_b[sb]));
+                    sp_commit(sp_smem_u32(&empty_a[sa]));
+                    sp_commit(sp_smem_u32(&empty_b[sb]));
                 }
-                sp_commit<kPair>(sp_smem_u32(&acc_full_bar));
+                sp_commit(sp_smem_u32(&acc_full_bar));
             }
             __syncwarp();
         } else if (warp == 3) {
@@ -616,7 +474,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             }
             __syncwarp();
         } else if (warp >= 4 && warp < 12) {
-            // ===== A builders: thread = pedestrian row; every row of every cell's (hi, lo) tile is written =====
+            // ===== A builders: thread = pedestrian row; every row of every cell's (hi, lo) vector is written =====
             const int bg = (warp - 4) >> 2;
             const uint32_t r = (uint32_t)((warp & 3) * 32 + lane);
             const int x = nsub == 2 ? bg : 0;                       // two tiles: builder group bg owns tile bg
@@ -624,15 +482,13 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             const bool row_ok = (int)r < nrows[x];
             const uint4* cr = row_ok ? reinterpret_cast<const uint4*>(p.cell_row + (size_t)row * p.cells) : nullptr;
             const int off_r = row_ok ? p.scene_off[p.row_scene[row]] - lbase[x] : 0;
-            // A stage of a two-tile round: [cell][tile][hi | lo]
-            unsigned char* a_ring = ring_ptr + (nsub == 2 ? (size_t)bg * 2u * kSpATile : 0u);
-            // TS: this warp's TMEM lane quarter, first column of the A ring (two tiles: [cell][tile][hi | lo])
+            // this warp's TMEM lane quarter, first column of the A ring (two tiles: [cell][tile][hi | lo])
             const uint32_t a_tmem = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + a_col0 + (nsub == 2 ? (uint32_t)bg * 16u : 0u);
 #define TB2_SP_BUILD(KCV, TWO)                                                                                          \
-    sp_builder<KCV, TWO, kTS>(cr, p.cells >> 4, a_ring, a_tmem, bg, r, off_r, nlat[x], latH[x], latL[x], empty_a, full_remote,  \
-                              lane, wait_e, SA, a_stage_cols)
-            if (nsub == 2) { if (wide_items) TB2_SP_BUILD(4, true); else if (kPair) TB2_SP_BUILD(2, true); else TB2_SP_BUILD(1, true); }
-            else { if (kPair) TB2_SP_BUILD(4, false); else TB2_SP_BUILD(2, false); }
+    sp_builder<KCV, TWO>(cr, p.cells >> 4, a_tmem, bg, off_r, nlat[x], latH[x], latL[x], empty_a, full_remote, lane, wait_e, \
+                         SA, a_stage_cols)
+            if (nsub == 2) { if (wide_items) TB2_SP_BUILD(4, true); else TB2_SP_BUILD(2, true); }
+            else TB2_SP_BUILD(4, false);
 #undef TB2_SP_BUILD
         }
         {
@@ -649,17 +505,16 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             auto chunk_col = [&](int ch, int& x) {           // first global hidden1 column of 16-column chunk ch, its piece
                 x = ch >= nchunk0 ? 1 : 0;
                 int dx = (x ? ch - nchunk0 : ch) * 16;                           // column inside the piece's accumulators
-                const int nrx = (int)ncols[x] / nC;                              // rows per CTA of the piece
+                const int nrx = (int)ncols[x] / 2;                               // rows per CTA of the piece
                 int gn = (int)ncols[x], goff = 0;                                // MMA group of this column
                 if (split) {
-                    if (dx >= 160) { dx -= 160; gn = (int)ncols[0] - 160; goff = 160 / nC; }
+                    if (dx >= 160) { dx -= 160; gn = (int)ncols[0] - 160; goff = 160 / 2; }
                     else gn = 160;
                 }
-                const int half = gn / nC;                                        // rows per CTA of the group
-                const int hsel = dx >= half ? 1 : 0;                             // which CTA's rows (pair only)
+                const int half = gn / 2;                                         // rows per CTA of the group
+                const int hsel = dx >= half ? 1 : 0;                             // which CTA's rows
                 return col0[x] + hsel * nrx + goff + (dx - hsel * half);
             };
-            if (p.w2 == nullptr) {
             for (int ch = sub; ch < nchunk; ch += 4) {
                 int x;
                 const int col = chunk_col(ch, x);
@@ -706,136 +561,13 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                 }
             }
             if (warp == 12 && lane == 0) t_epi_sum += clock64() - t_e0;
-            } else {
-            // ===== fused second Linear (reference gridbased_pooling.py:316-323, the 1024 -> 256 layer of two_layer):
-            // hidden1 = relu(b1 + D) never leaves the SM.  T1: the accumulators become A tiles (bf16 hi | lo, one tile
-            // pair per 16 columns = one k-step of layer 2) in the shared memory the rings used.  T2: the weight producer
-            // streams the matching k-step tiles of W2 (same pre-swizzled bulk-copy format as the layer-1 slabs), one
-            // thread issues D2[rows, 256] += A2_k . W2_k (3 passes) per k-step.  T3: D2, the piece's K-slice partial sum of
-            // the layer-2 pre-activation, goes to the partial buffer slot of the piece; pooled_reduce_kernel adds the
-            // slots of a tile in a fixed order, applies bias + ReLU and writes the gate kernel's operand. =====
-            unsigned char* a2 = ring_ptr;                                        // [chunk][hi tile | lo tile]
-            const uint32_t w_ring = ring + kSpA2Bytes;
-            const int TS = kPair ? kSpTailStages : 4;
-            const uint32_t w_stage = (uint32_t)(kSpN2 / nC) * 64u;               // this CTA's rows of one k-step tile
-            const uint32_t r_cta = (uint32_t)(q * 32 + lane);
-            for (int ch = sub; ch < nchunk; ch += 4) {
-                int x;
-                const int col = chunk_col(ch, x);
-                uint32_t v[16];
-                sp_tmem_ld16(trow + (uint32_t)(ch * 16), v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                uint32_t ph[8], pl[8];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float4 b4 = __ldg(reinterpret_cast<const float4*>(p.base + col) + i);
-                    const float bb[4] = {b4.x, b4.y, b4.z, b4.w};
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        const float x0 = fmaxf(__uint_as_float(v[4 * i + 2 * j]) + bb[2 * j], 0.f);
-                        const float x1 = fmaxf(__uint_as_float(v[4 * i + 2 * j + 1]) + bb[2 * j + 1], 0.f);
-                        const __nv_bfloat16 h0 = __float2bfloat16_rn(x0), h1 = __float2bfloat16_rn(x1);
-                        const __nv_bfloat16 l0 = __float2bfloat16_rn(x0 - __bfloat162float(h0));
-                        const __nv_bfloat16 l1 = __float2bfloat16_rn(x1 - __bfloat162float(h1));
-                        ph[2 * i + j] = (uint32_t)__bfloat16_as_ushort(h0) | ((uint32_t)__bfloat16_as_ushort(h1) << 16);
-                        pl[2 * i + j] = (uint32_t)__bfloat16_as_ushort(l0) | ((uint32_t)__bfloat16_as_ushort(l1) << 16);
-                    }
-                }
-                unsigned char* t = a2 + (size_t)ch * 2u * kSpATile;
-                *reinterpret_cast<uint4*>(t + sp_sw32(r_cta, 0)) = make_uint4(ph[0], ph[1], ph[2], ph[3]);
-                *reinterpret_cast<uint4*>(t + sp_sw32(r_cta, 1)) = make_uint4(ph[4], ph[5], ph[6], ph[7]);
-                *reinterpret_cast<uint4*>(t + kSpATile + sp_sw32(r_cta, 0)) = make_uint4(pl[0], pl[1], pl[2], pl[3]);
-                *reinterpret_cast<uint4*>(t + kSpATile + sp_sw32(r_cta, 1)) = make_uint4(pl[4], pl[5], pl[6], pl[7]);
-            }
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncthreads();
-            if (kPair) {      // both CTAs' A2 tiles are complete and their accumulators drained before the leader issues
-                asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-                asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-            }
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            if (warp == 0) {
-                if (lane == 0) {
-                    for (int ch = 0; ch < nchunk; ++ch) {
-                        int x;
-                        const int kstep = chunk_col(ch, x) >> 4;
-                        const uint32_t sw = (uint32_t)(ch % TS), pw = (uint32_t)((ch / TS) & 1);
-                        sp_mbar_wait(sp_smem_u32(&empty_w[sw]), pw ^ 1u);
-                        const uint32_t bar = sp_smem_u32(&full_w[sw]);
-                        sp_mbar_expect_tx(bar, w_stage);
-                        sp_bulk_load(w_ring + sw * w_stage, p.w2 + ((size_t)kstep * kSpN2 + rank * (uint32_t)(kSpN2 / nC)) * 64,
-                                     w_stage, bar);
-                    }
-                }
-                __syncwarp();
-            } else if (warp == 2) {
-                if (kPair && lane == 0 && rank != 0) {           // relay: "my tile of k-step ch has landed" -> leader
-                    for (int ch = 0; ch < nchunk; ++ch) {
-                        const uint32_t sw = (uint32_t)(ch % TS), pw = (uint32_t)((ch / TS) & 1);
-                        sp_mbar_wait(sp_smem_u32(&full_w[sw]), pw);
-                        uint32_t remote;
-                        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(remote) : "r"(sp_smem_u32(&peer_w[sw])), "r"(0));
-                        sp_mbar_arrive_cluster(remote);
-                    }
-                }
-                __syncwarp();
-            } else if (warp == 1) {
-                if (lane == 0 && rank == 0) {
-                    const uint32_t a_desc_hi = (uint32_t)(256 >> 4) | (1u << 14) | (6u << 29);
-                    const uint32_t b_desc_hi = (uint32_t)(512 >> 4) | (1u << 14) | (6u << 29);
-                    const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kSpN2 >> 3) << 17) | ((uint32_t)(R >> 4) << 24);
-                    for (int ch = 0; ch < nchunk; ++ch) {
-                        const uint32_t sw = (uint32_t)(ch % TS), pw = (uint32_t)((ch / TS) & 1);
-                        sp_mbar_wait(sp_smem_u32(&full_w[sw]), pw);
-                        if (kPair) sp_mbar_wait_cluster(sp_smem_u32(&peer_w[sw]), pw);
-                        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                        const int x = ch >= nchunk0 ? 1 : 0;
-                        const uint32_t d = tmem_base + (x ? (uint32_t)kSpN2 : 0u);
-                        const uint64_t ad = ((uint64_t)a_desc_hi << 32) | (uint64_t)(((ring + (uint32_t)ch * 2u * kSpATile) & 0x3FFFFu) >> 4);
-                        const uint64_t bd = ((uint64_t)b_desc_hi << 32) | (uint64_t)(((w_ring + sw * w_stage) & 0x3FFFFu) >> 4);
-                        const uint32_t first = (ch == 0 || ch == nchunk0) ? 0u : 1u;
-                        sp_umma<kPair>(d, ad, bd, idesc, first);                                // hi . hi
-                        sp_umma<kPair>(d, ad + (kSpATile >> 4), bd, idesc, 1u);                 // lo . hi
-                        sp_umma<kPair>(d, ad, bd + (256u >> 4), idesc, 1u);                     // hi . lo
-                        sp_commit<kPair>(sp_smem_u32(&empty_w[sw]));
-                    }
-                    sp_commit<kPair>(sp_smem_u32(&acc2_full_bar));
-                }
-                __syncwarp();
-            }
-            // T3: partial sums of the layer-2 pre-activation -> the slot of this piece
-            sp_mbar_wait(sp_smem_u32(&acc2_full_bar), 0u);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            for (int x = 0; x < nsub; ++x) {
-                const int row_t = (int)rank * 128 + q * 32 + lane;                // row inside the tile
-                const int slot = x ? rd.slot1 : rd.slot0;
-                float* dst = p.partials + (((size_t)tile[x] * p.max_slots + slot) * R + row_t) * kSpN2;
-                const bool row_ok = tile[x] * R + row_t < p.M;
-                for (int c16 = sub; c16 < kSpN2 / 16; c16 += 4) {
-                    uint32_t v[16];
-                    sp_tmem_ld16(trow + (uint32_t)(x * kSpN2 + c16 * 16), v);
-                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                    if (row_ok) {
-                        float4* d4 = reinterpret_cast<float4*>(dst + c16 * 16);
-#pragma unroll
-                        for (int i = 0; i < 4; ++i)
-                            d4[i] = make_float4(__uint_as_float(v[4 * i]), __uint_as_float(v[4 * i + 1]), __uint_as_float(v[4 * i + 2]),
-                                                __uint_as_float(v[4 * i + 3]));
-                    }
-                }
-            }
-            if (warp == 12 && lane == 0) t_epi_sum += clock64() - t_e0;
-            }
         }
         ++round_idx;
-        // the next round overwrites the latent tables, the TMEM accumulators and (pair) the peer's accumulators
+        // the next round overwrites the latent tables, the TMEM accumulators and the peer's accumulators
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
         __syncthreads();
-        if (kPair) {
-            asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-            asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-        }
+        asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+        asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     }
     if (dbg) {
@@ -852,8 +584,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
     }
     if (warp == 1) {
         uint32_t ncols = 512;
-        if (kPair) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
-        else asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
+        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
     }
 }
 
@@ -900,28 +631,27 @@ static bool plan_rounds_dp(long long total, int nb, int n_rounds, int cap, int c
     }
     const long long off_end = total - base(n_rounds) + W;
     if (off_end < 0 || off_end > 2 * W || from[n_rounds][(size_t)off_end] < 0) return false;
-    out.assign((size_t)n_rounds, SpRound{0, 0, 0, 0, 0, 0});
+    out.assign((size_t)n_rounds, SpRound{0, 0, 0, 0});
     long long end = total;
     for (int k = n_rounds; k > 0; --k) {
         const int sz = from[k][(size_t)(end - base(k) + W)];
         const long long pos = end - sz;
         const long long t0 = pos / nb;
         const long long in0 = std::min<long long>(sz, (t0 + 1) * nb - pos);
-        out[(size_t)k - 1] = SpRound{(int)t0, (int)(pos - t0 * nb), (int)in0, (int)(sz - in0), 0, 0};
+        out[(size_t)k - 1] = SpRound{(int)t0, (int)(pos - t0 * nb), (int)in0, (int)(sz - in0)};
         end = pos;
     }
     return end == 0;
 }
 
-// the round table of a (layout, OUT, units) combination lives with the layout (device memory of its device),
-// together with the partial-sum buffer of the fused second Linear and the number of pieces per tile
-static int get_plan(const tb2_layout* l, int OUT, int units_max, int nC, const tb2_layout::PairPlan** out, cudaStream_t st) {
+// the round table of a (layout, OUT, units) combination lives with the layout (device memory of its device)
+static int get_plan(const tb2_layout* l, int OUT, int units_max, const tb2_layout::PairPlan** out, cudaStream_t st) {
     static std::mutex mu;
     std::lock_guard<std::mutex> lock(mu);
     tb2_layout* lm = const_cast<tb2_layout*>(l);
     for (const auto& e : lm->pair_plans)
-        if (e.OUT == OUT && e.units_max == units_max && e.nC == nC) { *out = &e; return TB2_OK; }
-    const int R = 128 * nC, nb = OUT / 32;
+        if (e.OUT == OUT && e.units_max == units_max) { *out = &e; return TB2_OK; }
+    const int R = 256, nb = OUT / 32;                     // 256-row tiles (128 per CTA of a pair) x 32-column blocks
     const long long tiles = (l->M + R - 1) / R, total = tiles * nb;
     int units = units_max;
     if ((long long)units > total) units = (int)total;
@@ -929,92 +659,34 @@ static int get_plan(const tb2_layout* l, int OUT, int units_max, int nC, const t
     const int n_rounds = units * rpu;
     std::vector<SpRound> rounds;
     bool ok = false;       // smallest maximum round first (the kernel's time is the largest round), then the widest narrow piece
-    // a two-tile round moves twice the A tiles through shared memory (63 KB per cell against 43 KB: bound by the
-    // 128 B/clk port at ~490 cycles per cell instead of the 432-cycle tensor floor; measured 141-148 k cycles for 9
-    // blocks against 115 k): it gets one block less than the cap when the split allows it
+    // a two-tile round feeds two narrower accumulator chains and is slower per block than a one-tile round
+    // (DESIGN.md section 4.1): it gets one block less than the cap when the split allows it
     for (int cap = (int)((total + n_rounds - 1) / n_rounds); cap <= kSpMaxBlocks && !ok; ++cap)
         for (int relax = 0; relax < 2 && !ok; ++relax)
             for (int minpiece = 3; minpiece >= 1 && !ok; --minpiece)
                 ok = plan_rounds_dp(total, nb, n_rounds, cap, relax ? cap : std::max(cap - 1, 1), minpiece, rounds);
     if (!ok) { set_error("sparse_layer1_pair: no round plan (internal)"); return TB2_ERR_INVALID; }
-    // slot of every piece among the pieces of its tile (order of the rounds): pooled_reduce_kernel sums them in this order
-    std::vector<int> nslots((size_t)tiles, 0);
-    for (auto& r : rounds) {
-        if (r.n0 > 0) r.slot0 = nslots[(size_t)r.tile]++;
-        if (r.n1 > 0) r.slot1 = nslots[(size_t)r.tile + 1]++;
-    }
-    int max_slots = 1;
-    for (int v : nslots) max_slots = std::max(max_slots, v);
     SpRound* dev = nullptr;
-    int* dev_slots = nullptr;
-    float* partials = nullptr;
     TB2_CHECK_CUDA(cudaMalloc(&dev, rounds.size() * sizeof(SpRound)));
     lm->owned.push_back(dev);
-    TB2_CHECK_CUDA(cudaMalloc(&dev_slots, (size_t)tiles * sizeof(int)));
-    lm->owned.push_back(dev_slots);
-    TB2_CHECK_CUDA(cudaMalloc(&partials, (size_t)tiles * max_slots * R * kSpN2 * sizeof(float)));
-    lm->owned.push_back(partials);
     TB2_CHECK_CUDA(cudaMemcpyAsync(dev, rounds.data(), rounds.size() * sizeof(SpRound), cudaMemcpyHostToDevice, st));
-    TB2_CHECK_CUDA(cudaMemcpyAsync(dev_slots, nslots.data(), (size_t)tiles * sizeof(int), cudaMemcpyHostToDevice, st));
-    TB2_CHECK_CUDA(cudaStreamSynchronize(st));       // one-time (per layout): the host vectors are temporaries
+    TB2_CHECK_CUDA(cudaStreamSynchronize(st));       // one-time (per layout): the host vector is a temporary
     tb2_layout::PairPlan e;
-    e.OUT = OUT; e.units_max = units_max; e.nC = nC; e.units = units; e.rounds_per_unit = rpu; e.dev = dev;
-    e.tile_slots = dev_slots; e.partials = partials; e.max_slots = max_slots; e.R = R;
+    e.OUT = OUT; e.units_max = units_max; e.units = units; e.rounds_per_unit = rpu; e.dev = dev;
     lm->pair_plans.push_back(e);
     *out = &lm->pair_plans.back();
     return TB2_OK;
 }
 
-// pooled[row, :] = relu(b2 + sum over the tile's pieces (slot order) of partial[tile][slot][row, :]) -- the second Linear of
-// two_layer after the fused kernel; written as fp32 and / or as the bf16 (hi, lo) operand of the gate kernel
-__global__ void __launch_bounds__(256) pooled_reduce_kernel(const float* __restrict__ partials, const int* __restrict__ tile_slots,
-                                                            int max_slots, int R, int M, const float* __restrict__ bias,
-                                                            float* __restrict__ out, __nv_bfloat16* __restrict__ out_hi,
-                                                            __nv_bfloat16* __restrict__ out_lo) {
-    grid_dep_wait();
-    grid_dep_launch();
-    const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;            // one float4 of one row
-    if (idx >= (size_t)M * (kSpN2 / 4)) return;
-    const int row = (int)(idx / (kSpN2 / 4)), c4 = (int)(idx % (kSpN2 / 4)) * 4;
-    const int tile = row / R, rr = row - tile * R;
-    const int ns = tile_slots[tile];
-    const float4 b = *reinterpret_cast<const float4*>(bias + c4);
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-    for (int s = 0; s < ns; ++s) {
-        const float4 v = *reinterpret_cast<const float4*>(partials + (((size_t)tile * max_slots + s) * R + rr) * kSpN2 + c4);
-        acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
-    }
-    const float y[4] = {fmaxf(acc.x + b.x, 0.f), fmaxf(acc.y + b.y, 0.f), fmaxf(acc.z + b.z, 0.f), fmaxf(acc.w + b.w, 0.f)};
-    const size_t o = (size_t)row * kSpN2 + c4;
-    if (out) *reinterpret_cast<float4*>(out + o) = make_float4(y[0], y[1], y[2], y[3]);
-    if (out_hi) {
-        uint32_t ph[2], pl[2];
-#pragma unroll
-        for (int i = 0; i < 2; ++i) {
-            const __nv_bfloat16 h0 = __float2bfloat16_rn(y[2 * i]), h1 = __float2bfloat16_rn(y[2 * i + 1]);
-            const __nv_bfloat16 l0 = __float2bfloat16_rn(y[2 * i] - __bfloat162float(h0));
-            const __nv_bfloat16 l1 = __float2bfloat16_rn(y[2 * i + 1] - __bfloat162float(h1));
-            ph[i] = (uint32_t)__bfloat16_as_ushort(h0) | ((uint32_t)__bfloat16_as_ushort(h1) << 16);
-            pl[i] = (uint32_t)__bfloat16_as_ushort(l0) | ((uint32_t)__bfloat16_as_ushort(l1) << 16);
-        }
-        *reinterpret_cast<uint2*>(out_hi + o) = make_uint2(ph[0], ph[1]);
-        *reinterpret_cast<uint2*>(out_lo + o) = make_uint2(pl[0], pl[1]);
-    }
-}
-
-// fuse2: also run the second Linear (pool.embedding.2, 256 outputs) inside the kernel; `out*` then receive the POOLED
-// vector [M, 256] (fp32 and / or bf16 split) instead of hidden1
-template <bool kPair, bool kTS>
-static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float* out, void* out_hi,
-                                void* out_lo, bool fuse2, cudaStream_t st) {
-    constexpr int nC = kPair ? 2 : 1;
+int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float* out, void* out_hi, void* out_lo,
+                       cudaStream_t st) {
     static int sm_count[64] = {0};
     int dev = 0;
     TB2_CHECK_CUDA(cudaGetDevice(&dev));
     if (sm_count[dev & 63] == 0)
         TB2_CHECK_CUDA(cudaDeviceGetAttribute(&sm_count[dev & 63], cudaDevAttrMultiProcessorCount, dev));
     const int d1 = m->mlp_dims[1];
-    int units_max = sm_count[dev & 63] / nC;
+    int units_max = sm_count[dev & 63] / 2;
     {
         const char* e = getenv("TB2_PAIR_UNITS");      // debug knob
         if (e && atoi(e) > 0) units_max = atoi(e);
@@ -1022,14 +694,10 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
     SpParams p;
     const tb2_layout::PairPlan* plan = nullptr;
     int rc;
-    if ((rc = get_plan(l, d1, units_max, nC, &plan, st))) return rc;
+    if ((rc = get_plan(l, d1, units_max, &plan, st))) return rc;
     const int units = plan->units;
     p.rounds = (const SpRound*)plan->dev;
     p.rounds_per_unit = plan->rounds_per_unit;
-    p.w2 = fuse2 ? (const unsigned char*)m->W2_sw : nullptr;
-    p.partials = plan->partials;
-    p.N2 = kSpN2;
-    p.max_slots = plan->max_slots;
     p.scene_off = l->scene_off;
     p.row_scene = l->row_scene;
     p.cell_row = ws->cell_row;
@@ -1037,9 +705,9 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
     p.benc = m->benc;
     p.base = m->base1;
     p.w = (const unsigned char*)m->Wt1_sw_hi;
-    p.out = fuse2 ? nullptr : out;
-    p.out_hi = fuse2 ? nullptr : (__nv_bfloat16*)out_hi;
-    p.out_lo = fuse2 ? nullptr : (__nv_bfloat16*)out_lo;
+    p.out = out;
+    p.out_hi = (__nv_bfloat16*)out_hi;
+    p.out_lo = (__nv_bfloat16*)out_lo;
     p.M = l->M;
     p.OUT = d1;
     p.cells = m->cells;
@@ -1047,7 +715,7 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
     p.dbg = nullptr;
     static long long* dbg_buf = nullptr;
     static int dbg_calls = 0;
-    const int n_cta = units * nC;
+    const int n_cta = units * 2;
     {
         const char* e = getenv("TB2_L1_DEBUG");
         if (e && e[0] == '1') {
@@ -1058,9 +726,9 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
     const size_t smem = 1024 + kSpDynBytes + 64;
     static_assert(1024 + kSpDynBytes + 64 <= 227 * 1024 - 512, "shared memory budget");
     static DynSmemConfig configured;
-    TB2_CHECK_CUDA(configured.ensure(sparse_layer1_pair_kernel<kPair, kTS>, smem));
+    TB2_CHECK_CUDA(configured.ensure(sparse_layer1_pair_kernel, smem));
     {
-        KernelTimer kt(kPair ? (kTS ? "sparse_layer1_pair_ts" : "sparse_layer1_pair") : "sparse_layer1_solo", st);
+        KernelTimer kt("sparse_layer1_pair_ts", st);
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = dim3(n_cta);
         cfg.blockDim = dim3(kSpThreads);
@@ -1073,25 +741,16 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
             attr[na].val.programmaticStreamSerializationAllowed = 1;
             ++na;
         }
-        if (kPair) {
-            attr[na].id = cudaLaunchAttributeClusterDimension;
-            attr[na].val.clusterDim.x = 2;
-            attr[na].val.clusterDim.y = 1;
-            attr[na].val.clusterDim.z = 1;
-            ++na;
-        }
+        attr[na].id = cudaLaunchAttributeClusterDimension;
+        attr[na].val.clusterDim.x = 2;
+        attr[na].val.clusterDim.y = 1;
+        attr[na].val.clusterDim.z = 1;
+        ++na;
         cfg.attrs = attr;
         cfg.numAttrs = na;
-        TB2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, sparse_layer1_pair_kernel<kPair, kTS>, p));
+        TB2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, sparse_layer1_pair_kernel, p));
     }
     TB2_LAUNCH_CHECK();
-    if (fuse2) {
-        KernelTimer kt("pooled_reduce", st);
-        const unsigned blocks = (unsigned)(((size_t)l->M * (kSpN2 / 4) + 255) / 256);
-        launch_pdl(pooled_reduce_kernel, dim3(blocks), dim3(256), 0, st, (const float*)plan->partials, (const int*)plan->tile_slots,
-                   plan->max_slots, plan->R, l->M, (const float*)m->bl[1], out, (__nv_bfloat16*)out_hi, (__nv_bfloat16*)out_lo);
-        TB2_LAUNCH_CHECK();
-    }
     if (p.dbg && ++dbg_calls == 60) {
         std::vector<long long> h((size_t)n_cta * 8);
         cudaStreamSynchronize(st);
@@ -1107,55 +766,18 @@ static int launch_sparse_pair_t(const tb2_lstm* m, const tb2_layout* l, Workspac
             pdl += (double)(h[(size_t)c * 8 + 5] >> 24) / n_cta;
         }
         if (getenv("TB2_L1_DEBUG_ALL")) {
-            for (int c = 0; c < n_cta; c += nC) {
+            for (int c = 0; c < n_cta; c += 2) {
                 const long long* d = &h[(size_t)c * 8];
                 fprintf(stderr, "  unit %3d  last round blocks %2d + %2d | setup %6lld loop %7lld mma-wait %7lld epi %6lld total %7lld | builder: wait-empty %7lld wait-weights %7lld\n",
-                        c / nC, (int)(d[5] & 0xfff), (int)((d[5] >> 12) & 0xfff), d[0], d[1], d[2], d[3], d[6], d[4], d[7]);
+                        c / 2, (int)(d[5] & 0xfff), (int)((d[5] >> 12) & 0xfff), d[0], d[1], d[2], d[3], d[6], d[4], d[7]);
             }
         }
-        fprintf(stderr, "[tb2 sparse_pair x%d debug] per-CTA cycles: prologue + wait for the previous kernel %.0f | setup %.0f | cells loop until "
+        fprintf(stderr, "[tb2 sparse_pair x2 debug] per-CTA cycles: prologue + wait for the previous kernel %.0f | setup %.0f | cells loop until "
                         "accumulators ready %.0f | MMA thread waiting for A/B (leader CTAs, averaged over all) %.0f | epilogue %.0f | builder "
                         "warp 4: waiting for a free stage %.0f, for the weights %.0f | total after the wait %.0f (max %.0f) | SM clock "
                         "during the kernel (clock64 / globaltimer) %.3f GHz\n",
-                nC, pdl, a[0], a[1], a[2], a[3], a[4], a[7], a[6], mx, ghz);
+                pdl, a[0], a[1], a[2], a[3], a[4], a[7], a[6], mx, ghz);
     }
-    return TB2_OK;
-}
-
-// mode: 1 = one CTA per unit (cta_group::1), 2 = CTA pair (cta_group::2), 3 = CTA pair with the A operand in tensor memory
-int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, int mode, Workspace* ws, float* out, void* out_hi,
-                       void* out_lo, bool fuse2, cudaStream_t st) {
-    if (fuse2 && !(m->W2_sw != nullptr && m->n_mlp == 2 && m->mlp_dims[2] == kSpN2)) {
-        set_error("fused second Linear needs a two_layer embedding with 256 outputs");
-        return TB2_ERR_INVALID;
-    }
-    if (mode == 3) return launch_sparse_pair_t<true, true>(m, l, ws, out, out_hi, out_lo, fuse2, st);
-    if (mode == 2) return launch_sparse_pair_t<true, false>(m, l, ws, out, out_hi, out_lo, fuse2, st);
-    return launch_sparse_pair_t<false, false>(m, l, ws, out, out_hi, out_lo, fuse2, st);
-}
-
-bool sparse_pair_can_fuse(const tb2_lstm* m) { return m->W2_sw != nullptr && m->n_mlp == 2 && m->mlp_dims[2] == kSpN2; }
-
-// pool.embedding.2.weight [N2, K] -> bf16 [K / 16][N2 / 8][hi: 8 rows x 16 | lo: 8 rows x 16], 16-byte halves of a row
-// exchanged where ((n >> 2) & 1): the same bulk-copy image as the layer-1 slabs, one "slab" per k-step of layer 2
-__global__ void repack_layer2_sw_kernel(const float* __restrict__ W2, __nv_bfloat16* __restrict__ dst, int N2, int K) {
-    const size_t total = (size_t)N2 * K;
-    for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (size_t)gridDim.x * blockDim.x) {
-        const int n = (int)(idx / K), k = (int)(idx - (size_t)n * K);
-        const int kstep = k >> 4, c = k & 15;
-        const float v = W2[idx];
-        const __nv_bfloat16 h = __float2bfloat16_rn(v);
-        const int chunk = (c >> 3) ^ ((n >> 2) & 1);
-        const size_t atom = ((size_t)kstep * N2 + (size_t)(n & ~7)) * 32;          // bf16 elements: 8 rows x (hi 16 + lo 16)
-        const size_t e = atom + (size_t)(n & 7) * 16 + (size_t)(chunk * 8 + (c & 7));
-        dst[e] = h;
-        dst[e + 128] = __float2bfloat16_rn(v - __bfloat162float(h));
-    }
-}
-
-int launch_repack_layer2_sw(const float* W2, void* dst, int N2, int K, cudaStream_t st) {
-    repack_layer2_sw_kernel<<<512, 256, 0, st>>>(W2, (__nv_bfloat16*)dst, N2, K);
-    TB2_LAUNCH_CHECK();
     return TB2_OK;
 }
 

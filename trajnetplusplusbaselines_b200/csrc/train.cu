@@ -1487,7 +1487,7 @@ static int social_backward(const tb2_lstm* m, const tb2_layout* l, const tb2_lst
             TB2_LAUNCH_CHECK();
         } else {
         if ((rc = launch_pool_prepare(m, l, h_prev ? h_prev : b.zero_h, o1, o2, 1, 1, 0, &w2, st))) return rc;
-        if ((rc = launch_pool_mlp(m, l, &w2, ws.pooled, nullptr, nullptr, st, /*keep_hidden=*/true))) return rc;
+        if ((rc = launch_pool_mlp(m, l, &w2, ws.pooled, nullptr, nullptr, st))) return rc;
         if (two) {
             merge_split_kernel<<<1024, 256, 0, st>>>(tc2 ? (const __nv_bfloat16*)ws.act[0] : nullptr,
                                                      tc2 ? (const __nv_bfloat16*)ws.act[1] : nullptr, ws.act[0],
