@@ -302,17 +302,15 @@ int tb2_lstm_create(const tb2_lstm_config* cfg, tb2_lstm** out) {
         ALLOC(m->WgT[ph], (size_t)m->K_gate_pad * 4 * m->H);
         ALLOC(m->bg[ph], 4 * m->H);
     }
-    {
-        const char* no_tc = getenv("TB2_DISABLE_TC");
-        if (!(no_tc && no_tc[0] == '1') && gates_tc_supported(m)) {
-            const size_t half = ((size_t)4 * m->H * m->K_gate + 1) / 2;
-            for (int ph = 0; ph < 2; ++ph) {
-                float *hi, *lo;
-                ALLOC(hi, half);
-                ALLOC(lo, half);
-                m->Wg_hi[ph] = hi;
-                m->Wg_lo[ph] = lo;
-            }
+    const bool use_tc = !tc_disabled();
+    if (use_tc && gates_tc_supported(m)) {
+        const size_t half = ((size_t)4 * m->H * m->K_gate + 1) / 2;
+        for (int ph = 0; ph < 2; ++ph) {
+            float *hi, *lo;
+            ALLOC(hi, half);
+            ALLOC(lo, half);
+            m->Wg_hi[ph] = hi;
+            m->Wg_lo[ph] = lo;
         }
     }
     if (cfg->pool_type == TB2_POOL_SOCIAL) {
@@ -358,33 +356,28 @@ int tb2_lstm_create(const tb2_lstm_config* cfg, tb2_lstm** out) {
     if (m->n_mlp >= 1) {
         ALLOC(m->Wt1, (size_t)m->cells * m->C * m->mlp_dims[1]);
         ALLOC(m->base1, m->mlp_dims[1]);
-        {
-            const char* no_tc = getenv("TB2_DISABLE_TC");
-            if (cfg->pool_type == TB2_POOL_SOCIAL && m->C == 16 && !(no_tc && no_tc[0] == '1')) {
-                const size_t half = ((size_t)m->cells * 16 * m->mlp_dims[1] + 1) / 2;
-                float *hi, *lo;
-                ALLOC(hi, 2 * half);      // interleaved (hi | lo) slabs
-                ALLOC(lo, 4);
-                m->Wt1_hi = hi;
-                m->Wt1_lo = lo;
-                float *nh, *nl;
-                ALLOC(nh, half);
-                ALLOC(nl, half);
-                m->Wt1_nat_hi = nh;
-                m->Wt1_nat_lo = nl;
-                float *sh, *sl;
-                ALLOC(sh, 2 * half);      // hi and lo interleaved by 8-row group (one bulk copy per slab)
-                ALLOC(sl, 4);
-                m->Wt1_sw_hi = sh;
-                m->Wt1_sw_lo = sl;
-            }
+        if (cfg->pool_type == TB2_POOL_SOCIAL && m->C == 16 && use_tc) {
+            const size_t half = ((size_t)m->cells * 16 * m->mlp_dims[1] + 1) / 2;
+            float *hi, *lo;
+            ALLOC(hi, 2 * half);      // interleaved (hi | lo) slabs
+            ALLOC(lo, 4);
+            m->Wt1_hi = hi;
+            m->Wt1_lo = lo;
+            float *nh, *nl;
+            ALLOC(nh, half);
+            ALLOC(nl, half);
+            m->Wt1_nat_hi = nh;
+            m->Wt1_nat_lo = nl;
+            float *sh, *sl;
+            ALLOC(sh, 2 * half);      // hi and lo interleaved by 8-row group (one bulk copy per slab)
+            ALLOC(sl, 4);
+            m->Wt1_sw_hi = sh;
+            m->Wt1_sw_lo = sl;
         }
         for (int layer = 1; layer < m->n_mlp; ++layer) {
             ALLOC(m->WT[layer], (size_t)m->mlp_dims[layer] * m->mlp_dims[layer + 1]);
             ALLOC(m->bl[layer], m->mlp_dims[layer + 1]);
-            // TB2_DISABLE_TC=1: debug knob for A/B parity runs (fp32 FFMA layer instead of tcgen05)
-            const char* no_tc = getenv("TB2_DISABLE_TC");
-            if (layer == 1 && !(no_tc && no_tc[0] == '1') && dense_tc_supported(m->mlp_dims[1], m->mlp_dims[2])) {
+            if (layer == 1 && use_tc && dense_tc_supported(m->mlp_dims[1], m->mlp_dims[2])) {
                 const size_t half = ((size_t)m->mlp_dims[1] * m->mlp_dims[2] + 1) / 2;   // bf16 pairs in float units
                 float *hi, *lo;
                 ALLOC(hi, half);

@@ -54,6 +54,13 @@ inline bool pdl_enabled() {
     return on;
 }
 
+// TB2_DISABLE_TC=1: fp32 FFMA kernels instead of the tensor-core ones, for parity runs of the tcgen05 path.  Read
+// when a model is created (its weights are laid out for one path or the other).
+inline bool tc_disabled() {
+    const char* e = getenv("TB2_DISABLE_TC");
+    return e && e[0] == '1';
+}
+
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                               Args&&... args) {

@@ -19,9 +19,6 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <math_constants.h>
-#include <cstdio>
-#include <cstdlib>
-#include <vector>
 
 #include "common.cuh"
 
@@ -112,7 +109,6 @@ struct GateTcParams {
     const float* Wn;            // [5, 128]
     const float* bn;            // [5]
     int M, P;
-    long long* dbg;             // optional [grid, 8] cycle stamps (TB2_GATES_DEBUG=1)
 };
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kGtThreads, 1)
@@ -137,8 +133,6 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
     const int kb_pool = p.P / kGtBK;       // k-blocks: [emb | pooled x kb_pool | h x 2]
     const int num_kb = 1 + kb_pool + 2;
     const uint32_t ring = (g_smem_u32(smem_gt) + 1023u) & ~1023u;
-    long long* dbg = p.dbg ? p.dbg + (size_t)(blockIdx.y * 2 + blockIdx.x) * 8 : nullptr;
-    const long long t_begin = clock64();
 
     for (int i = threadIdx.x; i < 5 * 64; i += kGtThreads) wn_s[i / 64][i % 64] = p.Wn[(i / 64) * kGtH + rank * 64 + (i % 64)];
     for (int i = threadIdx.x; i < 4 * 64; i += kGtThreads) bg_s[i / 64][i % 64] = p.bg[(i / 64) * kGtH + rank * 64 + (i % 64)];
@@ -162,7 +156,6 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
     const uint32_t tmem_base = tmem_base_slot;
     grid_dep_wait();          // embedding / pooled / state operands come from the previous kernels
     grid_dep_launch();
-    if (dbg && threadIdx.x == 0) dbg[0] = clock64() - t_begin;
     // cluster barrier phase 1 (arrive now, wait before the first DSMEM access): a CTA may only
     // touch its peer's shared memory once the peer is known to be resident
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -197,13 +190,10 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
         if (lane == 0) {
             const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(kGtBN >> 3) << 17) |
                                    ((uint32_t)(kGtBM >> 4) << 24);
-            long long wait_tma = 0;
             for (int kb = 0; kb < num_kb; ++kb) {
                 const int s = kb % kGtStages;
                 const uint32_t phase = (kb / kGtStages) & 1;
-                const long long tw = clock64();
                 g_mbar_wait(g_smem_u32(&full_bar[s]), phase);
-                wait_tma += clock64() - tw;
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t base = ring + s * kGtStageBytes;
                 const uint64_t a_hi = g_umma_desc(base);
@@ -220,7 +210,6 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
                 g_umma_commit(g_smem_u32(&empty_bar[s]));
             }
             g_umma_commit(g_smem_u32(&tmem_full_bar));
-            if (dbg) { dbg[1] = clock64() - t_begin; dbg[2] = wait_tma; }
         }
         __syncwarp();
     } else {
@@ -233,7 +222,6 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
         row_masked = isnan(o1.x) || isnan(o2.x);                             // lstm.py:118
         g_mbar_wait(g_smem_u32(&tmem_full_bar), 0);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        if (dbg && warp == 2 && lane == 0) dbg[3] = clock64() - t_begin;
         const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
         // All MMAs have retired, so the operand ring is free: each epilogue warp stages its
         // [32 rows x 16 units] tiles of c and h there, so that global loads / stores run with
@@ -334,12 +322,10 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
                 asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(remote + 4 * o), "f"(part[o]) : "memory");
         }
     }
-    if (dbg && warp == 2 && lane == 0) dbg[4] = clock64() - t_begin;
     // cluster barrier phase 2: rank 1's partial sums are visible in rank 0's shared memory afterwards
     if (!waited_phase1) asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
     asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-    if (dbg && warp == 2 && lane == 0) dbg[5] = clock64() - t_begin;
     if (warp >= 2 && warp < 6 && rank == 0 && row_valid) {
         const int rl = (warp & 3) * 32 + lane;
         float* no = p.normal_out + (size_t)row * 5;
@@ -365,7 +351,6 @@ lstm_gates_tc_kernel(const __grid_constant__ CUtensorMap map_emb_hi, const __gri
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (dbg && threadIdx.x == 0) dbg[6] = clock64() - t_begin;
     if (warp == 1) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kGtTmemCols) : "memory");
     }
@@ -492,17 +477,6 @@ int launch_gates_tc(const tb2_lstm* m, const tb2_layout* l, int phase, const flo
     p.bn = m->bn;
     p.M = M;
     p.P = m->P;
-    p.dbg = nullptr;
-    static long long* dbg_buf = nullptr;
-    static int dbg_calls = 0;
-    const int n_cta = 2 * ((M + kGtBM - 1) / kGtBM);
-    {
-        const char* e = getenv("TB2_GATES_DEBUG");
-        if (e && e[0] == '1') {
-            if (!dbg_buf) cudaMalloc(&dbg_buf, (size_t)n_cta * 8 * sizeof(long long));
-            p.dbg = dbg_buf;
-        }
-    }
     const size_t smem = (size_t)kGtStages * kGtStageBytes + 1024;
     static DynSmemConfig configured;
     TB2_CHECK_CUDA(configured.ensure(lstm_gates_tc_kernel, smem));
@@ -513,16 +487,6 @@ int launch_gates_tc(const tb2_lstm* m, const tb2_layout* l, int phase, const flo
                    mw_hi, mw_lo, p);
     }
     TB2_LAUNCH_CHECK();
-    if (p.dbg && ++dbg_calls == 60) {
-        std::vector<long long> h((size_t)n_cta * 8);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        double a[7] = {0, 0, 0, 0, 0, 0, 0};
-        for (int c = 0; c < n_cta; ++c) for (int k = 0; k < 7; ++k) a[k] += (double)h[(size_t)c * 8 + k] / n_cta;
-        fprintf(stderr, "[tb2 gates_tc debug] per-CTA cycles since start: setup %.0f | mma issued %.0f (waited on TMA %.0f) | "
-                        "acc ready %.0f | epilogue done %.0f | cluster barrier %.0f | end %.0f\n",
-                a[0], a[1], a[2], a[3], a[4], a[5], a[6]);
-    }
     return TB2_OK;
 }
 

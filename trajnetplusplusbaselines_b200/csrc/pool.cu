@@ -11,10 +11,8 @@
 #include <cuda_bf16.h>
 #include <math_constants.h>
 #include <algorithm>
-#include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <vector>
 
 #include "common.cuh"
 
@@ -86,7 +84,6 @@ struct PrepParams {
     int E;
     int n_max, H, C, n, pool_type, front, skip_masked, write_pairs, pad_to_max;
     float side, width;
-    long long* dbg;           // optional [B, 8] clock64 stamps (TB2_PREP_DEBUG=1)
 };
 
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
@@ -133,8 +130,6 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
     }
     grid_dep_wait();          // obs / hidden state come from the previous kernels of the stream
     grid_dep_launch();
-    long long* dbg = p.dbg ? p.dbg + (size_t)blockIdx.x * 8 : nullptr;
-    const long long t_begin = clock64();
 
     if (fast_lat) {           // raw rows (nan_to_num is applied where they are read), asynchronously
         const float* hsrc = p.hidden + (size_t)row0 * 128;
@@ -159,7 +154,6 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
     }
     cp_async_wait_all();
     __syncthreads();
-    if (dbg && tid == 0) dbg[0] = clock64() - t_begin;
     if (p.emb_hi != nullptr) {
         // emb = cat(relu(W_e . (4 v) + b_e), 0, 0) (modules.py:24-30) as bf16 (hi, lo) for the gate GEMM
         const int e_shift = (p.E & (p.E - 1)) == 0 ? 31 - __clz(p.E) : -1;       // E = 64: no integer division per element
@@ -174,7 +168,6 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
             p.emb_lo[(size_t)(row0 + j) * p.E + k] = __float2bfloat16_rn(e - __bfloat162float(h));
         }
     }
-    if (dbg && tid == 0) dbg[1] = clock64() - t_begin;
     if (fast_lat) {
         // lat[j][c] = sum_k nan_to_num(h[j][k]) * WencT[k][c] + benc[c]: one warp per pedestrian, lane = (4 channels,
         // 16-wide k slice); the slice sums are added across the 8 slices by an xor tree (fixed order)
@@ -234,7 +227,6 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
         return;
     }
 
-    if (dbg && tid == 0) dbg[2] = clock64() - t_begin;
     const float offx = p.width * 0.5f;
     const float offy = p.front ? 0.f : p.width * 0.5f;
     int* myrow = cellrow + warp * nm1;
@@ -274,7 +266,6 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
             }
         }
         __syncwarp();
-        if (dbg && warp == 0 && lane == 0 && i == 0) dbg[5] = clock64() - t_begin;
         // pass 2: winners, compacted in ascending jj
         const bool masked = isnan(vi.x);      // obs2 - obs1 is NaN iff the track is absent at either frame
         int count = 0;
@@ -320,9 +311,7 @@ __global__ void __launch_bounds__(kPrepMaxThreads, 2) pool_prepare_kernel(PrepPa
         }
         if (lane == 0) p.win_count[row0 + i] = count;
         __syncwarp();
-        if (dbg && warp == 0 && lane == 0 && i == 0) dbg[6] = clock64() - t_begin;
     }
-    if (dbg && lane == 0 && warp == 0) dbg[3] = clock64() - t_begin;
 }
 
 int launch_pool_prepare(const tb2_lstm* m, const tb2_layout* l, const float* hidden,
@@ -358,16 +347,6 @@ int launch_pool_prepare(const tb2_lstm* m, const tb2_layout* l, const float* hid
     p.E = m->E;
     p.emb_hi = write_emb ? (__nv_bfloat16*)ws->emb_hi : nullptr;
     p.emb_lo = write_emb ? (__nv_bfloat16*)ws->emb_lo : nullptr;
-    p.dbg = nullptr;
-    static long long* dbg_buf = nullptr;
-    static int dbg_calls = 0;
-    {
-        const char* e = getenv("TB2_PREP_DEBUG");
-        if (e && e[0] == '1') {
-            if (!dbg_buf) cudaMalloc(&dbg_buf, (size_t)4096 * 8 * sizeof(long long));
-            if (l->B <= 4096 && l->B >= 64) p.dbg = dbg_buf;        // the BASELINE-size batches only
-        }
-    }
     p.side = m->cfg.cell_side;        // pool_size == 1
     p.width = (float)m->cfg.n;
     int nm1 = l->n_max > 1 ? l->n_max - 1 : 1;
@@ -383,16 +362,6 @@ int launch_pool_prepare(const tb2_lstm* m, const tb2_layout* l, const float* hid
         launch_pdl(pool_prepare_kernel, dim3(l->B), dim3(nthreads), smem, st, p);
     }
     TB2_LAUNCH_CHECK();
-    if (p.dbg && ++dbg_calls == 60) {
-        std::vector<long long> h((size_t)l->B * 8);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        double a[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        for (int c = 0; c < l->B; ++c) for (int k = 0; k < 8; ++k) a[k] += (double)h[(size_t)c * 8 + k] / l->B;
-        fprintf(stderr, "[tb2 pool_prepare debug] per-CTA cycles since start (after the dependency wait): staged %.0f | emb %.0f | "
-                        "lat %.0f | winners: row 0 binned %.0f, row 0 done %.0f, warp 0 done %.0f\n",
-                a[0], a[1], a[2], a[5], a[6], a[3]);
-    }
     return TB2_OK;
 }
 
@@ -654,7 +623,6 @@ struct L1MmaParams {
     __nv_bfloat16* out_lo;
     int OUT, cells, nm1, cap, relu;
     float constant;
-    long long* dbg;               // optional [grid, 8] clock64 phase stamps (TB2_L1_DEBUG=1)
 };
 
 constexpr int kMmaThreads = 256;          // 8 warps x 32 output columns
@@ -667,8 +635,6 @@ __global__ void __launch_bounds__(kMmaThreads, 1) sparse_layer1_mma_kernel(L1Mma
     const int row0 = p.scene_off[s0];
     const int P = p.scene_off[s1] - row0;
     const int chunk0 = blockIdx.y * kL1Cols;
-    long long* dbg = p.dbg ? p.dbg + (size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 8 : nullptr;
-    if (dbg && tid == 0) dbg[0] = clock64();
 
     // acc rows [0, cap) real, [cap, cap + 16) dummies absorbing the padding rows of an MMA tile;
     // lat rows [0, cap) real, cap = NaN-padded slot (b_enc), cap + 1 = zeros (padding rows)
@@ -746,7 +712,6 @@ __global__ void __launch_bounds__(kMmaThreads, 1) sparse_layer1_mma_kernel(L1Mma
         }
     }
     __syncthreads();
-    if (dbg && tid == 0) dbg[1] = clock64();
 
     // padding rows of a tile: zero latent row, per-lane dummy accumulator rows
     const uint32_t dummy0 = ((uint32_t)(p.cap + 1) << 16) | (uint32_t)(p.cap + g);
@@ -828,9 +793,7 @@ __global__ void __launch_bounds__(kMmaThreads, 1) sparse_layer1_mma_kernel(L1Mma
             if (cell + 7 < nc) b3 = load_b(phys(cell + 7));
         }
     }
-    if (dbg && lane == 0) dbg[2 + (warp & 3)] = clock64();      // main loop end of warps 0..3
     __syncthreads();
-    if (dbg && tid == 0) dbg[6] = clock64();
     {
         const int col = chunk0 + tid;
         if (col < p.OUT) {
@@ -848,7 +811,6 @@ __global__ void __launch_bounds__(kMmaThreads, 1) sparse_layer1_mma_kernel(L1Mma
             }
         }
     }
-    if (dbg && tid == 0) dbg[7] = clock64();
 }
 
 static size_t l1_mma_smem_bytes(int cap, int cells, int nm1) {
@@ -1206,15 +1168,6 @@ int launch_pool_mlp(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float
         q.base = m->base1; q.out = p.out; q.out_hi = p.out_hi; q.out_lo = p.out_lo;
         q.OUT = d1; q.cells = m->cells; q.nm1 = nm1; q.cap = l->group_cap[gm]; q.relu = 1;
         q.constant = m->cfg.constant;
-        q.dbg = nullptr;
-        static long long* dbg_buf = nullptr;
-        static int dbg_calls = 0;
-        const char* dbgenv = getenv("TB2_L1_DEBUG");
-        const int n_cta = l->num_groups[gm] * ((d1 + kL1Cols - 1) / kL1Cols);
-        if (dbgenv && dbgenv[0] == '1') {
-            if (!dbg_buf) cudaMalloc(&dbg_buf, (size_t)n_cta * 8 * sizeof(long long));
-            q.dbg = dbg_buf;
-        }
         static DynSmemConfig configured;
         TB2_CHECK_CUDA(configured.ensure(sparse_layer1_mma_kernel, sm));
         dim3 grid(l->num_groups[gm], (d1 + kL1Cols - 1) / kL1Cols);
@@ -1223,20 +1176,6 @@ int launch_pool_mlp(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, float
             sparse_layer1_mma_kernel<<<grid, kMmaThreads, sm, st>>>(q);
         }
         TB2_LAUNCH_CHECK();
-        if (q.dbg && ++dbg_calls == 60) {       // one warm launch, printed once
-            std::vector<long long> hbuf((size_t)n_cta * 8);
-            cudaStreamSynchronize(st);
-            cudaMemcpy(hbuf.data(), dbg_buf, hbuf.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-            double setup = 0, loop = 0, tail = 0, epi = 0;
-            for (int c = 0; c < n_cta; ++c) {
-                const long long* d = &hbuf[(size_t)c * 8];
-                long long lmax = std::max(std::max(d[2], d[3]), std::max(d[4], d[5]));
-                long long lmin = std::min(std::min(d[2], d[3]), std::min(d[4], d[5]));
-                setup += d[1] - d[0]; loop += lmin - d[1]; tail += lmax - lmin; epi += d[7] - d[6];
-            }
-            fprintf(stderr, "[tb2 l1 debug] per-CTA cycles: setup %.0f  main loop (fastest of 4 warps) %.0f  "
-                            "spread %.0f  epilogue %.0f\n", setup / n_cta, loop / n_cta, tail / n_cta, epi / n_cta);
-        }
         rc = TB2_OK;
     } else
     switch (m->cfg.pool_type) {

@@ -38,8 +38,6 @@
 // one tile each); all 16 warps run the epilogue (4 per TMEM lane quarter).
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <cstdio>
-#include <cstdlib>
 #include <algorithm>
 #include <mutex>
 #include <vector>
@@ -146,7 +144,6 @@ struct SpParams {
     const SpRound* rounds;           // [units * rounds_per_unit] (plan_rounds)
     int M, OUT, cells, rounds_per_unit;
     float constant;
-    long long* dbg;                  // optional [2 * units, 8] cycle counters (TB2_L1_DEBUG=1)
 };
 
 // MMA with A = 128 lanes x 8 TMEM columns (16 bf16 of K per lane) of each CTA, B from shared memory (64-bit
@@ -190,7 +187,7 @@ __device__ __forceinline__ void sp_build_item(uint32_t a_item, uint32_t cell_col
 template <int KC, bool kTwo>
 __device__ __forceinline__ void sp_builder(const uint4* cr, int groups, uint32_t a_tmem, int bg, int off_r, int nlat,
                                            const uint4* lh, const uint4* ll, uint64_t* empty_a,
-                                           const uint32_t (&full_remote)[kSpSA], int lane, long long& wait_e,
+                                           const uint32_t (&full_remote)[kSpSA], int lane,
                                            uint32_t SA, uint32_t stage_cols) {
     static_assert(kTwo || KC == 4, "one-tile rounds use 4-cell items");
     const uint4 none = make_uint4(~0u, ~0u, ~0u, ~0u);
@@ -212,9 +209,7 @@ __device__ __forceinline__ void sp_builder(const uint4* cr, int groups, uint32_t
                 bytes = jj == 0 ? (bg ? cur.y : cur.x) : (bg ? cur.w : cur.z);
             }
             const uint32_t sa = g % SA, pa = (g / SA) & 1u;
-            const long long tw0 = clock64();
             sp_mbar_wait(sp_smem_u32(&empty_a[sa]), pa ^ 1u);
-            wait_e += clock64() - tw0;
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             sp_build_item<KC>(a_tmem + sa * stage_cols, kTwo ? 32u : 16u, bytes, off_r, nlat, lh, ll);
             asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
@@ -240,8 +235,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
     uint32_t rank;
     asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
     const int unit = (int)(blockIdx.x >> 1);
-    long long* dbg = p.dbg ? p.dbg + (size_t)blockIdx.x * 8 : nullptr;
-    const long long t_begin = clock64();
 
     const uint32_t ring = (sp_smem_u32(smem_sp) + 1023u) & ~1023u;          // weight ring
     unsigned char* ring_ptr = smem_sp + (ring - sp_smem_u32(smem_sp));
@@ -263,8 +256,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = tmem_base_slot;
-    long long t_start = 0;
-    unsigned long long ns_start = 0;
 
     // leader's full barrier as seen from this CTA (cluster address space)
     uint32_t full_remote[kSpSA];
@@ -275,12 +266,9 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
     }
 
     uint32_t round_idx = 0;
-    long long t_setup_sum = 0, t_loop_sum = 0, t_epi_sum = 0, wait_full = 0, wait_b = 0, wait_e = 0;
-    SpRound rd = {0, 0, 0, 0};
     for (int ri = 0; ri < p.rounds_per_unit; ++ri) {
-        rd = p.rounds[(size_t)unit * p.rounds_per_unit + ri];
+        const SpRound rd = p.rounds[(size_t)unit * p.rounds_per_unit + ri];
         if (rd.n0 == 0) continue;                         // padding round (uniform for the whole cluster)
-        const long long t_r0 = clock64();
         const int nsub = rd.n1 > 0 ? 2 : 1;
         // pipeline shape of the round (the barriers are re-initialised for it)
         // two-tile round of <= 256 accumulator columns: items of 4 cells of both tiles (one barrier round trip per
@@ -344,8 +332,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
         if (round_idx == 0) {
             grid_dep_wait();          // cell map / latent vectors come from pool_prepare
             grid_dep_launch();
-            t_start = clock64();
-            if (dbg) asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns_start));
         }
         // ---- round setup (all warps): split latent tables of the one / two tiles ---------------------
         int rbase[2], nrows[2], lbase[2], nlat[2];
@@ -381,8 +367,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
         // the peer's barriers must be initialised before the first remote arrive / multicast commit
         asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
         asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-        const long long t_r1 = clock64();
-        t_setup_sum += t_r1 - (round_idx == 0 ? t_start : t_r0);
 
         // MMA groups of a one-tile round: a 9-block piece is issued as N = 160 + 128 over the same A operand
         const bool split = ncols[0] > 256u;
@@ -430,9 +414,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                 for (int it = 0; it < n_items; ++it) {
                     const uint32_t sa = (uint32_t)it % SA, pa = ((uint32_t)it / SA) & 1u;
                     const uint32_t sb = (uint32_t)it % SB;
-                    const long long t0 = clock64();
                     sp_mbar_wait_cluster(sp_smem_u32(&full_a[sa]), pa);
-                    wait_full += clock64() - t0;
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     if (have) {
                         // A from tensor memory: stage sa, (two tiles: the issuer's own tile inside every cell)
@@ -466,9 +448,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                     const uint32_t sa = (uint32_t)it % SA, pa = ((uint32_t)it / SA) & 1u;
                     const uint32_t sb = (uint32_t)it % SB, pb = ((uint32_t)it / SB) & 1u;
                     sp_mbar_wait(sp_smem_u32(&empty_a[sa]), pa ^ 1u);
-                    const long long tw1 = clock64();
                     sp_mbar_wait(sp_smem_u32(&full_b[sb]), pb);
-                    wait_b += clock64() - tw1;
                     sp_mbar_arrive_cluster(full_remote[sa]);
                 }
             }
@@ -485,7 +465,7 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             // this warp's TMEM lane quarter, first column of the A ring (two tiles: [cell][tile][hi | lo])
             const uint32_t a_tmem = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + a_col0 + (nsub == 2 ? (uint32_t)bg * 16u : 0u);
 #define TB2_SP_BUILD(KCV, TWO)                                                                                          \
-    sp_builder<KCV, TWO>(cr, p.cells >> 4, a_tmem, bg, off_r, nlat[x], latH[x], latL[x], empty_a, full_remote, lane, wait_e, \
+    sp_builder<KCV, TWO>(cr, p.cells >> 4, a_tmem, bg, off_r, nlat[x], latH[x], latL[x], empty_a, full_remote, lane,    \
                          SA, a_stage_cols)
             if (nsub == 2) { if (wide_items) TB2_SP_BUILD(4, true); else TB2_SP_BUILD(2, true); }
             else TB2_SP_BUILD(4, false);
@@ -496,8 +476,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
             const int q = warp & 3, sub = warp >> 2;
             sp_mbar_wait(sp_smem_u32(&acc_full_bar), 0u);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const long long t_e0 = clock64();
-            if (warp == 12 && lane == 0) t_loop_sum += t_e0 - t_r1;
             const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16);
             // accumulator column d of an MMA group = row (d mod n/2) of the slab of CTA (d div n/2): 16-column
             // chunks never straddle the two halves (n/2 is a multiple of 16)
@@ -560,7 +538,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
                     }
                 }
             }
-            if (warp == 12 && lane == 0) t_epi_sum += clock64() - t_e0;
         }
         ++round_idx;
         // the next round overwrites the latent tables, the TMEM accumulators and the peer's accumulators
@@ -569,18 +546,6 @@ __global__ void __launch_bounds__(kSpThreads, 1) sparse_layer1_pair_kernel(SpPar
         asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
         asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    }
-    if (dbg) {
-        if (tid == 0) {
-            unsigned long long ns_end;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ns_end));
-            dbg[0] = t_setup_sum | ((long long)(ns_end - ns_start) << 24); dbg[6] = clock64() - t_start;
-            dbg[5] = (long long)rd.n0 | ((long long)rd.n1 << 12) | ((long long)(t_start - t_begin) << 24);
-        }
-        if (warp == 1 && lane == 0) dbg[2] = wait_full;
-        if (warp == 4 && lane == 0) dbg[4] = wait_e;
-        if (warp == 3 && lane == 0) dbg[7] = wait_b;
-        if (warp == 12 && lane == 0) { dbg[1] = t_loop_sum; dbg[3] = t_epi_sum; }
     }
     if (warp == 1) {
         uint32_t ncols = 512;
@@ -686,11 +651,7 @@ int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, fl
     if (sm_count[dev & 63] == 0)
         TB2_CHECK_CUDA(cudaDeviceGetAttribute(&sm_count[dev & 63], cudaDevAttrMultiProcessorCount, dev));
     const int d1 = m->mlp_dims[1];
-    int units_max = sm_count[dev & 63] / 2;
-    {
-        const char* e = getenv("TB2_PAIR_UNITS");      // debug knob
-        if (e && atoi(e) > 0) units_max = atoi(e);
-    }
+    const int units_max = sm_count[dev & 63] / 2;
     SpParams p;
     const tb2_layout::PairPlan* plan = nullptr;
     int rc;
@@ -712,17 +673,6 @@ int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, fl
     p.OUT = d1;
     p.cells = m->cells;
     p.constant = m->cfg.constant;
-    p.dbg = nullptr;
-    static long long* dbg_buf = nullptr;
-    static int dbg_calls = 0;
-    const int n_cta = units * 2;
-    {
-        const char* e = getenv("TB2_L1_DEBUG");
-        if (e && e[0] == '1') {
-            if (!dbg_buf) { cudaMalloc(&dbg_buf, (size_t)1024 * 8 * sizeof(long long)); cudaMemset(dbg_buf, 0, (size_t)1024 * 8 * sizeof(long long)); }
-            if (n_cta <= 1024) p.dbg = dbg_buf;
-        }
-    }
     const size_t smem = 1024 + kSpDynBytes + 64;
     static_assert(1024 + kSpDynBytes + 64 <= 227 * 1024 - 512, "shared memory budget");
     static DynSmemConfig configured;
@@ -730,7 +680,7 @@ int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, fl
     {
         KernelTimer kt("sparse_layer1_pair_ts", st);
         cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3(n_cta);
+        cfg.gridDim = dim3(2 * units);
         cfg.blockDim = dim3(kSpThreads);
         cfg.dynamicSmemBytes = smem;
         cfg.stream = st;
@@ -751,33 +701,6 @@ int launch_sparse_pair(const tb2_lstm* m, const tb2_layout* l, Workspace* ws, fl
         TB2_CHECK_CUDA(cudaLaunchKernelEx(&cfg, sparse_layer1_pair_kernel, p));
     }
     TB2_LAUNCH_CHECK();
-    if (p.dbg && ++dbg_calls == 60) {
-        std::vector<long long> h((size_t)n_cta * 8);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        double a[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-        double mx = 0, pdl = 0, ghz = 0;
-        for (int c = 0; c < n_cta; ++c) {
-            const long long ns = h[(size_t)c * 8] >> 24;
-            h[(size_t)c * 8] &= 0xffffff;
-            if (ns > 0) ghz += (double)h[(size_t)c * 8 + 6] / (double)ns / n_cta;
-            for (int k = 0; k < 8; ++k) a[k] += (double)h[(size_t)c * 8 + k] / n_cta;
-            if ((double)h[(size_t)c * 8 + 6] > mx) mx = (double)h[(size_t)c * 8 + 6];
-            pdl += (double)(h[(size_t)c * 8 + 5] >> 24) / n_cta;
-        }
-        if (getenv("TB2_L1_DEBUG_ALL")) {
-            for (int c = 0; c < n_cta; c += 2) {
-                const long long* d = &h[(size_t)c * 8];
-                fprintf(stderr, "  unit %3d  last round blocks %2d + %2d | setup %6lld loop %7lld mma-wait %7lld epi %6lld total %7lld | builder: wait-empty %7lld wait-weights %7lld\n",
-                        c / 2, (int)(d[5] & 0xfff), (int)((d[5] >> 12) & 0xfff), d[0], d[1], d[2], d[3], d[6], d[4], d[7]);
-            }
-        }
-        fprintf(stderr, "[tb2 sparse_pair x2 debug] per-CTA cycles: prologue + wait for the previous kernel %.0f | setup %.0f | cells loop until "
-                        "accumulators ready %.0f | MMA thread waiting for A/B (leader CTAs, averaged over all) %.0f | epilogue %.0f | builder "
-                        "warp 4: waiting for a free stage %.0f, for the weights %.0f | total after the wait %.0f (max %.0f) | SM clock "
-                        "during the kernel (clock64 / globaltimer) %.3f GHz\n",
-                pdl, a[0], a[1], a[2], a[3], a[4], a[7], a[6], mx, ghz);
-    }
     return TB2_OK;
 }
 

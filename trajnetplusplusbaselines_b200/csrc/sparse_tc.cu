@@ -22,9 +22,6 @@
 // 4..11 = epilogue (lane quarter = warp % 4, column block = (warp - 4) / 4), 3, 12, 13 = more builders.
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <cstdio>
-#include <cstdlib>
-#include <vector>
 
 #include "common.cuh"
 
@@ -107,7 +104,6 @@ struct ScParams {
     __nv_bfloat16* out_lo;
     int OUT, cells, nm1, cap;
     float constant;
-    long long* dbg;              // optional [grid, 8] cycle counters (TB2_L1_DEBUG=1)
 };
 
 // byte offset of (row r, 16-byte chunk c) inside a SWIZZLE_32B K-major tile
@@ -129,8 +125,6 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
     const int P = p.scene_off[s1] - row0;
     const int Npad = (P + 15) & ~15;
     const int chunk0 = blockIdx.y * kScCols;
-    long long* dbg = p.dbg ? p.dbg + (size_t)(blockIdx.y * gridDim.x + blockIdx.x) * 8 : nullptr;
-    const long long t_begin = clock64();
 
     const uint32_t ring = (sc_smem_u32(smem_sc) + 1023u) & ~1023u;
     unsigned char* ring_ptr = smem_sc + (ring - sc_smem_u32(smem_sc));
@@ -238,7 +232,6 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         setup_sync();
     }
-    const long long t_setup = clock64();
 
     if (warp == 0) {
         // ===== TMA producer: weight slabs of the non-empty cells =====
@@ -262,16 +255,11 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
         // ===== MMA issuer =====
         if (lane == 0) {
             const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(Npad >> 3) << 17) | (8u << 24);
-            long long wait_a = 0, wait_b = 0;
             for (int it = 0; it < n_items; ++it) {
                 const int s = it % kScStages;
                 const uint32_t ph = (it / kScStages) & 1;
-                const long long t0 = clock64();
                 sc_mbar_wait(sc_smem_u32(&full_a[s]), ph);
-                const long long t1 = clock64();
                 sc_mbar_wait(sc_smem_u32(&full_b[s]), ph);
-                wait_a += t1 - t0;
-                wait_b += clock64() - t1;
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 const uint32_t base = ring + s * kScStageBytes;
                 const uint64_t b_hi = sc_umma_desc(base + 4 * kScABytes);
@@ -288,7 +276,6 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
                 sc_umma_commit(sc_smem_u32(&empty_bar[s]));
             }
             sc_umma_commit(sc_smem_u32(&acc_full_bar));
-            if (dbg) { dbg[0] = t_setup - t_begin; dbg[1] = clock64() - t_setup; dbg[2] = wait_a; dbg[3] = wait_b; dbg[4] = n_items; }
         }
         __syncwarp();
     } else if (warp == 2 || warp == 3 || warp >= 12) {
@@ -332,7 +319,6 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
         const int col = chunk0 + blk * 128 + q * 32 + lane;
         sc_mbar_wait(sc_smem_u32(&acc_full_bar), 0);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        if (dbg && warp == 4 && lane == 0) dbg[5] = clock64() - t_setup;
         const float b = col < p.OUT ? p.base[col] : 0.f;
         const uint32_t trow = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(blk * 256);
         for (int p0 = 0; p0 < Npad; p0 += 16) {
@@ -365,7 +351,6 @@ sparse_layer1_tc_kernel(const __grid_constant__ CUtensorMap map_w_hi, const __gr
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if (dbg && tid == 0) dbg[6] = clock64() - t_begin;
     if (warp == 1) {
         uint32_t ncols = 512;
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(ncols) : "memory");
@@ -442,17 +427,6 @@ int launch_sparse_tc(const tb2_lstm* m, const tb2_layout* l, int gsel, Workspace
     p.nm1 = nm1;
     p.cap = l->group_cap[gsel];
     p.constant = m->cfg.constant;
-    p.dbg = nullptr;
-    static long long* dbg_buf = nullptr;
-    static int dbg_calls = 0;
-    const int n_cta = l->num_groups[gsel] * (d1 / kScCols);
-    {
-        const char* e = getenv("TB2_L1_DEBUG");
-        if (e && e[0] == '1') {
-            if (!dbg_buf) cudaMalloc(&dbg_buf, (size_t)n_cta * 8 * sizeof(long long));
-            p.dbg = dbg_buf;
-        }
-    }
     const size_t smem = sparse_tc_smem_bytes(p.cap, m->cells, nm1);
     static DynSmemConfig configured;
     TB2_CHECK_CUDA(configured.ensure(sparse_layer1_tc_kernel, smem));
@@ -462,15 +436,6 @@ int launch_sparse_tc(const tb2_lstm* m, const tb2_layout* l, int gsel, Workspace
         launch_pdl(sparse_layer1_tc_kernel, grid, dim3(kScThreads), smem, st, mh, ml, p);
     }
     TB2_LAUNCH_CHECK();
-    if (p.dbg && ++dbg_calls == 60) {
-        std::vector<long long> h((size_t)n_cta * 8);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(h.data(), dbg_buf, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        double a[7] = {0, 0, 0, 0, 0, 0, 0};
-        for (int c = 0; c < n_cta; ++c) for (int k = 0; k < 7; ++k) a[k] += (double)h[(size_t)c * 8 + k] / n_cta;
-        fprintf(stderr, "[tb2 sparse_tc debug] per-CTA cycles: setup %.0f | mma loop %.0f (wait TMA %.0f, wait builder %.0f, "
-                        "items %.0f) | acc ready at %.0f | total %.0f\n", a[0], a[1], a[2], a[3], a[4], a[5], a[6]);
-    }
     return TB2_OK;
 }
 

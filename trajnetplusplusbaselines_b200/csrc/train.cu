@@ -1054,7 +1054,7 @@ static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 
 // Large plain GEMMs of the all-row (social) backward: cuBLAS with FP32 emulation on the bf16 tensor cores
 // (CUBLAS_COMPUTE_32F_EMULATED_16BFX9: every fp32 operand is split into three bf16 values, nine products,
 // fp32-accurate) -- library code for plain library GEMMs; everything with a gather, a mask or a fused epilogue
-// stays in the kernels of this file.  TB2_CUBLAS=0 forces the FFMA kernels (A/B), =2 plain fp32 cuBLAS.
+// stays in the kernels of this file.  Where a cuBLAS build rejects the emulated mode, plain fp32 cuBLAS is used.
 // ------------------------------------------------------------------------------------------
 // cuBLAS is bound at run time (dlopen): inside a torch process the already loaded libcublas.so.12 is used, whatever
 // its minor version; entry points a build does not have (cublasSetEmulationStrategy) are simply skipped, and without
@@ -1084,24 +1084,17 @@ static const CublasApi& cublas_api() {
     return api;
 }
 
-static cublasHandle_t cublas_for_device(int* mode_out) {
+static cublasHandle_t cublas_for_device() {
+    if (!cublas_api().ok) return nullptr;
     static std::mutex mu;
     static cublasHandle_t handles[64] = {nullptr};
-    static int mode = -1;            // 0 off, 1 emulated bf16x9, 2 fp32
     std::lock_guard<std::mutex> lock(mu);
-    if (mode < 0) {
-        const char* e = getenv("TB2_CUBLAS");
-        mode = e ? atoi(e) : 1;
-        if (mode != 0 && !cublas_api().ok) mode = 0;
-    }
-    *mode_out = mode;
-    if (mode == 0) return nullptr;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
     cublasHandle_t& h = handles[dev & 63];
     if (!h) {
         if (cublas_api().create(&h) != CUBLAS_STATUS_SUCCESS) { h = nullptr; return nullptr; }
-        if (mode == 1 && cublas_api().set_emulation) cublas_api().set_emulation(h, CUBLAS_EMULATION_STRATEGY_EAGER);
+        if (cublas_api().set_emulation) cublas_api().set_emulation(h, CUBLAS_EMULATION_STRATEGY_EAGER);
     }
     return h;
 }
@@ -1110,8 +1103,7 @@ static cublasHandle_t cublas_for_device(int* mode_out) {
 static bool cublas_gemm(cublasOperation_t ta, cublasOperation_t tb, int m, int n, int k, const float* A, int lda,
                         const float* B, int ldb, float beta, float* C, int ldc, const char* name, cudaStream_t st) {
     if ((double)m * n * k < 3.2e7) return false;            // small problems: the FFMA kernels (deterministic split order)
-    int mode = 0;
-    cublasHandle_t h = cublas_for_device(&mode);
+    cublasHandle_t h = cublas_for_device();
     if (!h) return false;
     const CublasApi& api = cublas_api();
     static bool emulation_ok = true;
@@ -1119,7 +1111,7 @@ static bool cublas_gemm(cublasOperation_t ta, cublasOperation_t tb, int m, int n
     KernelTimer kt(name, st);
     if (api.set_stream(h, st) != CUBLAS_STATUS_SUCCESS) return false;
     cublasStatus_t rc = CUBLAS_STATUS_NOT_SUPPORTED;
-    if (mode == 1 && emulation_ok) {
+    if (emulation_ok) {
         rc = api.gemm_ex(h, ta, tb, m, n, k, &alpha, A, CUDA_R_32F, lda, B, CUDA_R_32F, ldb, &beta, C, CUDA_R_32F, ldc,
                          CUBLAS_COMPUTE_32F_EMULATED_16BFX9, CUBLAS_GEMM_DEFAULT);
         if (rc != CUBLAS_STATUS_SUCCESS) emulation_ok = false;
@@ -1401,8 +1393,7 @@ static size_t carve_social(const tb2_lstm* m, const tb2_layout* l, size_t S, voi
 template <int C>
 static int social_pair_kernels(const tb2_lstm* m, const tb2_layout* l, const SocBuffers& b, const float* lat,
                                int nm1, int d1, cudaStream_t st) {
-    const char* nomma = getenv("TB2_DGRID_FFMA");               // A/B knob: the fp32 FFMA kernel
-    if (C == 16 && d1 % 32 == 0 && b.Wt1_hi != nullptr && dgrid_mma_smem(d1) <= 200 * 1024 && !(nomma && nomma[0] == '1')) {
+    if (C == 16 && d1 % 32 == 0 && b.Wt1_hi != nullptr && dgrid_mma_smem(d1) <= 200 * 1024) {
         static DynSmemConfig configured;
         TB2_CHECK_CUDA(configured.ensure(social_dgrid_mma_kernel, dgrid_mma_smem(d1), 48 * 1024));
         KernelTimer kt("social_dgrid_mma", st);
@@ -1414,7 +1405,7 @@ static int social_pair_kernels(const tb2_lstm* m, const tb2_layout* l, const Soc
             b.sorted, b.start, b.DH1, d1, m->Wt1, nm1, b.DGRID);
     }
     TB2_LAUNCH_CHECK();
-    if (C == 16 && d1 % 32 == 0 && !(nomma && nomma[0] == '1')) {
+    if (C == 16 && d1 % 32 == 0) {
         KernelTimer kt("social_dw1_mma", st);
         social_dw1_mma_kernel<<<dim3(m->cells, (d1 + 255) / 256), 256, 0, st>>>(
             b.sorted, b.start, nm1, l->row_scene, l->scene_off, lat, b.DH1, d1, b.dWt1);
@@ -1486,14 +1477,14 @@ static int social_backward(const tb2_lstm* m, const tb2_layout* l, const tb2_lst
                                                     M * P);
             TB2_LAUNCH_CHECK();
         } else {
-        if ((rc = launch_pool_prepare(m, l, h_prev ? h_prev : b.zero_h, o1, o2, 1, 1, 0, &w2, st))) return rc;
-        if ((rc = launch_pool_mlp(m, l, &w2, ws.pooled, nullptr, nullptr, st))) return rc;
-        if (two) {
-            merge_split_kernel<<<1024, 256, 0, st>>>(tc2 ? (const __nv_bfloat16*)ws.act[0] : nullptr,
-                                                     tc2 ? (const __nv_bfloat16*)ws.act[1] : nullptr, ws.act[0],
-                                                     b.H1 + (size_t)s * M * d1, M * d1);
-            TB2_LAUNCH_CHECK();
-        }
+            if ((rc = launch_pool_prepare(m, l, h_prev ? h_prev : b.zero_h, o1, o2, 1, 1, 0, &w2, st))) return rc;
+            if ((rc = launch_pool_mlp(m, l, &w2, ws.pooled, nullptr, nullptr, st))) return rc;
+            if (two) {
+                merge_split_kernel<<<1024, 256, 0, st>>>(tc2 ? (const __nv_bfloat16*)ws.act[0] : nullptr,
+                                                         tc2 ? (const __nv_bfloat16*)ws.act[1] : nullptr, ws.act[0],
+                                                         b.H1 + (size_t)s * M * d1, M * d1);
+                TB2_LAUNCH_CHECK();
+            }
         }
         {
             KernelTimer kt("bwd_gather", st);
@@ -1506,9 +1497,8 @@ static int social_backward(const tb2_lstm* m, const tb2_layout* l, const tb2_lst
     }
     // The row GEMMs (rows = all tracks) run on the 3-pass tcgen05 kernel of the forward (dense_layer_tc_kernel:
     // Y = A . W^T + bias, bf16 (hi, lo) operands, fp32 accumulation) when the shapes allow it: A and the (transposed)
-    // weights are split once, the outputs stay fp32.  TB2_BWD_TC=0: cuBLAS / FFMA GEMMs (A/B).
-    const char* notc = getenv("TB2_BWD_TC");
-    const bool tcg = !(notc && notc[0] == '0') && K == EP + 128 && dense_tc_supported(K, 512) && dense_tc_supported(512, 128) &&
+    // weights are split once, the outputs stay fp32.  Other shapes: cuBLAS / FFMA GEMMs.
+    const bool tcg = K == EP + 128 && dense_tc_supported(K, 512) && dense_tc_supported(512, 128) &&
                      dense_tc_supported(512, EP) && (!two || dense_tc_supported(P, d1));
     if (tcg) {
         TB2_CHECK_CUDA(cudaMemsetAsync(b.zero_bias, 0, (size_t)(d1 > 512 ? d1 : 512) * sizeof(float), st));
@@ -1677,12 +1667,6 @@ static int social_backward(const tb2_lstm* m, const tb2_layout* l, const tb2_lst
             return rc;
     }
     if ((rc = colsum(b.DLAT, C, S * Mi, C, g->pool_encoding_bias, nullptr, b.scratch, b.scratch_floats, st))) return rc;
-    if (const char* dump = getenv("TB2_DUMP_DLAT")) {       // debug: d lat of every (step, track) as raw fp32 [S, M, C]
-        std::vector<float> host((size_t)S * M * C);
-        cudaStreamSynchronize(st);
-        cudaMemcpy(host.data(), b.DLAT, host.size() * sizeof(float), cudaMemcpyDeviceToHost);
-        if (FILE* f = fopen(dump, "wb")) { fwrite(host.data(), sizeof(float), host.size(), f); fclose(f); }
-    }
     return TB2_OK;
 }
 }  // namespace tb2
